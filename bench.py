@@ -213,6 +213,8 @@ def main():
     ap.add_argument("--ref-time-limit", type=float, default=450.0,
                     help="reference arm: HiGHS limit per MILP (s); measured on one core: 120-190 s per config-D scenario, 192 s for a "
                          "fallback scenario (two MILPs), so the whole arm ends within a few minutes")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (rank 0), to compare two builds")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -309,6 +311,8 @@ def main():
         ksolve.append(tm["ms_solve"]); kplace.append(tm["ms_place"])
         nfb += int(res["status"] == 1); shortf += int(res["shortfall"])
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, rem_mc, xm, bm, nr)
     if world > 1:
         dist.barrier()
     eng.set_option(8, 0)
@@ -423,6 +427,20 @@ def main():
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, res, rem, xm, bm, nr):
+    """The last timed step as a caller of it receives it: the Monte-Carlo mean remaining runtimes the solve planned with
+    (remaining_runtime [J]), the round and back-fill schedules unpacked from their 128-bit masks (x, backfill [J, T]),
+    the rounds per job (nrounds [J]) and the solve's result record (result: the swb_result fields in declaration order)."""
+    from shockwave_b200.engine import Result, unpack_masks
+    os.makedirs(out_dir, exist_ok=True)
+    masks = lambda t: unpack_masks(t[0].cpu().numpy().view(np.uint64), T).astype(np.float32)
+    arrays = {"remaining_runtime": rem[0].cpu().numpy().astype(np.float64), "x": masks(xm), "backfill": masks(bm),
+              "nrounds": nr[0].cpu().numpy().astype(np.float32),
+              "result": np.array([float(res[f]) for f, _ in Result._fields_], dtype=np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def cpu_baseline_sample():

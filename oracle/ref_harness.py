@@ -12,9 +12,8 @@ generated gRPC stubs are absent.  This module
      and returns the same result dictionary that script pickles.
 
 Nothing here is imported by the product; it exists to (a) pin the oracle against the reference's
-golden pickles and (b) record solver-input fixtures for the GPU parity tests.  It works where /root/reference
-exists (this container) or where oracle/stage_ref.py staged the reference files (baseline/_ref, untracked, shipped to
-the GPU box by gpurun).
+golden pickles and (b) record solver-input fixtures for the GPU parity tests.  It works where the reference's
+scheduler/ directory exists or where build() made its byte-compiled copy under oracle/_ref (see oracle/stage_ref.py).
 """
 from __future__ import annotations
 
@@ -31,9 +30,9 @@ _ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 def _find_ref():
     """The reference's scheduler/ directory: $SWB_REF_SCHEDULER, else /root/reference (build container), else the
-    byte-for-byte staged copy under baseline/_ref (git-ignored, shipped to the GPU box; see oracle/stage_ref.py)."""
+    byte-compiled build under oracle/_ref (git-ignored, made by build(); see oracle/stage_ref.py)."""
     for cand in (os.environ.get("SWB_REF_SCHEDULER"), "/root/reference/scheduler",
-                 os.path.join(_ROOT, "baseline", "_ref", "scheduler")):
+                 os.path.join(_ROOT, "oracle", "_ref", "scheduler")):
         if cand and os.path.isdir(cand):
             return cand
     return "/root/reference/scheduler"

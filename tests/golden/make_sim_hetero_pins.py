@@ -7,7 +7,7 @@ makespan, rounds.  oracle/sim_loop.py and the host build of sim_core.cuh replay 
 reproduce these numbers exactly (tests/test_oracle_sim_hetero.py); the device loop does the same on the B200
 (tests/test_zz_gpu_sim_hetero.py).
 
-    python -m tests.golden.make_sim_hetero_pins         (needs /root/reference or the staged copy under baseline/_ref)
+    python -m tests.golden.make_sim_hetero_pins         (needs the reference's scheduler/ directory or its build under oracle/_ref)
 """
 import json
 import os

@@ -5,7 +5,7 @@ trace as plain arrays, the per-round schedule the reference chose, and what the 
 completion times, makespan, the measured-throughput timeline of every job (`_throughput_timeline`, scheduler.py:549-571).
 The restatement oracle/sim_loop.py replays the recorded schedules and must reproduce these numbers exactly.
 
-    python -m tests.golden.make_sim_pins         (needs /root/reference or the staged copy under baseline/_ref)
+    python -m tests.golden.make_sim_pins         (needs the reference's scheduler/ directory or its build under oracle/_ref)
 """
 import json
 import math

@@ -3,9 +3,8 @@ ShockwaveScheduler / Gavel policies — libswb200.so in the loop — on the cano
 (reproduce/tacc_32gpus.sh), end-to-end metrics against the golden pickles the reference ships (within the 3 % spread of
 its own three Shockwave pickles, BASELINE.md §2).
 
-Needs a B200 AND the reference's python files.  The build container has /root/reference but no GPU; the GPU box gets
-the byte-for-byte staged copy `baseline/_ref/scheduler` (git-ignored, made by `python -m oracle.stage_ref`, shipped by
-gpurun like a pip --target install of the reference would be).  Every run appends its metrics to
+Needs a B200 AND the reference's simulator: the reference's scheduler/ directory, or the byte-compiled build of it that
+build() makes under oracle/_ref/scheduler (git-ignored, `python -m oracle.stage_ref`).  Every run appends its metrics to
 gpurun_out/closed_loop.json (copied to profiles/closed_loop_rNN.json for the record)."""
 import glob
 import json

@@ -1,10 +1,7 @@
 """The numpy restatement of the forecast (oracle/jobmeta.py) against the reference's own JobMetaData:
  (a) through the committed fixture — values the reference objects produced inside the canonical
      simulation, replayed solve by solve (stateful calibration + share series included);
- (b) directly, when /root/reference is importable (this container only)."""
-import os
-import sys
-
+ (b) directly, on random job histories, against the values the reference's JobMetaData computed for them."""
 import numpy as np
 import pytest
 
@@ -29,43 +26,24 @@ def test_replay_matches_reference_recorded_forecast():
     assert worst["dbar"] <= 1e-9 and worst["rem"] <= 1e-9 and worst["ftobj"] <= 1e-9
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not os.path.isdir("/root/reference/scheduler"), reason="needs /root/reference")
 def test_direct_against_reference_jobmetadata():
-    sys.path.insert(0, "/root/reference/scheduler")
-    try:
-        from JobMetaData import JobMetaData
-    finally:
-        sys.path.pop(0)
+    """The restatement on 40 random job histories against what the reference's JobMetaData computed on the same
+    histories (tests/golden/make_jobmeta_pins.py)."""
     from collections import OrderedDict
-    rng = np.random.default_rng(0)
-    for trial in range(40):
-        E = int(rng.integers(3, 60))
-        nm = int(rng.integers(1, 4))
-        modes = rng.choice([16, 32, 64, 128, 256], size=nm, replace=False)
-        bs = np.sort(rng.choice(modes, size=E))
-        dur = rng.uniform(5, 400, size=E)
-        prof = dict(model="ResNet-18", dataset="CIFAR-10", num_samples_per_epoch=50000, num_epochs=E,
-                    util_every_epoch=[1.0] * E, mem_every_epoch=[1000.0] * E,
-                    duration_every_epoch=dur.tolist(), scale_factor=int(rng.choice([1, 2, 4])),
-                    bs_every_epoch=[int(b) for b in bs])
-        ref = JobMetaData(trial, prof)
+    from tests.golden import make_jobmeta_pins as pins
+    recs = pins.load()
+    for (trial, prof, steps), rec in zip(pins.histories(), recs):
+        E = prof["num_epochs"]
         tl = OrderedDict()
-        ref.register_job_submit(123.0)
-        ref.set_throughput_measurments(tl, 120)
-        mine = ojm.JobState(trial, ref.nworkers, E, 50000, ref.epoch_duration_preprofiled, ref.bs_schedule, 123.0, 120)
+        mine = ojm.JobState(trial, rec["nworkers"], E, 50000, rec["pre"], rec["bs"], 123.0, 120)
         mine.timeline = tl
-        rnd = 0
-        for step in range(12):
-            c = int(rng.integers(0, E + 1))
-            ref.set_epoch_progress(c); mine.epoch_progress = c
-            if rng.random() < 0.7:
-                rnd += int(rng.integers(1, 4))
-                tl[rnd] = (float(rng.uniform(0.2, 30.0)), int(rng.choice(modes)))
-            ref.calibrate_profiled_epoch_duration(); mine.calibrate()
-            assert np.isclose(mine.elapsed(), sum(ref.epoch_duration[:c]), rtol=1e-12)
-            a, b = ref.dirichlet_posterior_remaining_runtime(), mine.remaining()
-            assert np.isclose(a, b, rtol=1e-12), (trial, step, a, b)
-            ref.calibrate_profiled_epoch_duration()
-            a = float(np.mean(ref.epoch_duration[: c + 1]))
-            assert np.isclose(a, mine.interpolate_epoch_duration(), rtol=1e-12)
+        for (c, entry), (elapsed, remaining, interp) in zip(steps, rec["values"]):
+            mine.epoch_progress = c
+            if entry is not None:
+                tl[entry[0]] = entry[1]
+            mine.calibrate()
+            assert np.isclose(mine.elapsed(), elapsed, rtol=1e-12)
+            b = mine.remaining()
+            assert np.isclose(remaining, b, rtol=1e-12), (trial, c, remaining, b)
+            assert np.isclose(interp, mine.interpolate_epoch_duration(), rtol=1e-12)
+    assert len(recs) == 40

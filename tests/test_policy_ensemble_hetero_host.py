@@ -1,20 +1,19 @@
 """Host logic of shockwave_b200.simulate.PolicyEnsemble on MIXED clusters (several worker types, static jobs) against the
-UNMODIFIED reference loop (CPU): the same policy code with the HiGHS backend behind it runs (a) inside the reference's
-Scheduler.simulate() on a v100 + p100 + k80 cluster and (b) inside the ensemble driver, on the host build of the device
-loop with the oracle restatement of the round step.  Identical per-round schedules (jobs AND worker ids, same insertion
-order), completion times and makespan mean the driver keeps the per-worker-type time accounting, deficits, worker-id
-layout and the order the types are walked in (incl. the reference's type shuffler for the policies without `Perf` in
-their name) exactly as scheduler.py:1290-1301, :1826-1832, :3498-3551, :3611-3724, :4660-4672 do."""
+UNMODIFIED reference loop (CPU): the same policy code with the HiGHS backend behind it ran (a) inside the reference's
+Scheduler.simulate() on a v100 + p100 + k80 cluster (recorded by tests/golden/make_loop_records.py) and runs (b) inside
+the ensemble driver, on the host build of the device loop with the oracle restatement of the round step.  Identical
+per-round schedules (jobs AND worker ids, same insertion order), completion times and makespan mean the driver keeps the
+per-worker-type time accounting, deficits, worker-id layout and the order the types are walked in (incl. the reference's
+type shuffler for the policies without `Perf` in their name) exactly as scheduler.py:1290-1301, :1826-1832, :3498-3551,
+:3611-3724, :4660-4672 do."""
 import numpy as np
 import pytest
 
 from oracle import gavel_backend as gb
-from oracle import ref_harness as rh
 from oracle import sim_loop
 from oracle.gavel_round_backend import OracleBackend
 from tests import sim_fixtures as sf_
-
-pytestmark = pytest.mark.skipif(not rh.reference_available(), reason="staged reference not present")
+from tests.golden import make_loop_records as records
 
 
 @pytest.mark.parametrize("policy,keep,cluster", [("max_min_fairness_perf", 40, "4:3:2"), ("finish_time_fairness_perf", 36, "2:4:4"),
@@ -24,8 +23,7 @@ def test_policy_ensemble_on_a_mixed_cluster_equals_the_reference_loop(monkeypatc
     if sf_.host_sim_lib() is None:
         pytest.skip("g++ not available")
     from shockwave_b200 import simulate as sim
-    from tests.golden import make_sim_hetero_pins as gen
-    rec = gen.record(policy, keep, cluster)
+    rec = records.load("hetero", policy, keep, cluster)
     tr = sim_loop.trace_arrays(rec)
     wt = dict(names=rec["worker_types"], throughput=np.asarray(rec["throughput_w"]), ngpus=rec["ngpus_w"])
     with gb.cpu_backend() as P:

@@ -24,10 +24,12 @@ def _inputs():
     return tr, profiles
 
 
-def _patch():
+def _patch(set_=setattr):
+    """CPU stand-ins for the device loop and the solver: `set_` is monkeypatch.setattr in the pytest process (undone
+    after the test, so later GPU tests get the device classes back), plain setattr in a spawned rank."""
     from shockwave_b200 import simulate as sim
-    sim.DeviceSim = sf_.HostDeviceSim
-    sim.ShockwaveScheduler = sf_.make_rule_scheduler_cls()
+    set_(sim, "DeviceSim", sf_.HostDeviceSim)
+    set_(sim, "ShockwaveScheduler", sf_.make_rule_scheduler_cls())
     return sim
 
 
@@ -47,7 +49,7 @@ def _worker(rank, world, port, q):
     dist.destroy_process_group()
 
 
-def test_two_rank_sharded_sweep_equals_the_single_process_run():
+def test_two_rank_sharded_sweep_equals_the_single_process_run(monkeypatch):
     if sf_.host_sim_lib() is None:
         pytest.skip("g++ not available")
     import torch.multiprocessing as tmp
@@ -60,7 +62,7 @@ def test_two_rank_sharded_sweep_equals_the_single_process_run():
     res = sorted([q.get(timeout=300) for _ in range(2)], key=lambda t: t[0])
     for p in procs:
         p.join(timeout=60)
-    sim = _patch()
+    sim = _patch(monkeypatch.setattr)
     tr, profiles = _inputs()
     one = sim.run_sharded(tr, profiles, CFG, SCEN, 8, device=0)
     assert sim.shard_scenarios(5, 0, 2) == [0, 2, 4] and sim.shard_scenarios(5, 1, 2) == [1, 3]
@@ -85,10 +87,10 @@ def _policy_inputs():
     return tr, wt
 
 
-def _run_policies(rank, world, gather):
+def _run_policies(rank, world, gather, set_=setattr):
     from oracle import gavel_backend as gb
     from oracle.gavel_round_backend import OracleBackend
-    sim = _patch()
+    sim = _patch(set_)
     tr, wt = _policy_inputs()
     with gb.cpu_backend() as P:
         P.set_device = lambda d: None                      # no engine on the CPU stand-ins
@@ -116,7 +118,7 @@ def _policy_worker(rank, world, port, q):
     dist.destroy_process_group()
 
 
-def test_two_rank_sharded_policy_sweep_equals_the_single_process_run():
+def test_two_rank_sharded_policy_sweep_equals_the_single_process_run(monkeypatch):
     if sf_.host_sim_lib() is None:
         pytest.skip("g++ not available")
     import torch.multiprocessing as tmp
@@ -129,7 +131,7 @@ def test_two_rank_sharded_policy_sweep_equals_the_single_process_run():
     res = sorted([q.get(timeout=300) for _ in range(2)], key=lambda t: t[0])
     for p in procs:
         p.join(timeout=60)
-    one = _run_policies(0, 1, None)
+    one = _run_policies(0, 1, None, monkeypatch.setattr)
     assert np.isfinite(one["makespan"]).all()
     for _, makespan, jct, rounds, sched in res:
         assert np.array_equal(makespan, one["makespan"]) and np.array_equal(rounds, one["rounds"])
