@@ -166,7 +166,7 @@ __global__ void __launch_bounds__(SWB_PLACE_THREADS, 1) place_kernel(PlaceLaunch
   if (J <= SWB_SMEM_JOBS) {
     xm = reinterpret_cast<unsigned long long *>(p);
     bm = xm + 2 * (size_t)J;
-    rr_smem = p + 32 * (size_t)J;
+    if (L.rr_hot_smem) rr_smem = p + 32 * (size_t)J;
   } else {
     xm = gmask + (size_t)s * 4 * J;
     bm = xm + 2 * (size_t)J;
@@ -937,15 +937,17 @@ cudaError_t launch_place(const PlaceLaunch &L, cudaStream_t st, unsigned long lo
   }
   int nt = npad < SWB_PLACE_THREADS ? npad : SWB_PLACE_THREADS;
   // re-rank search: its hot arrays (w_j, one dense (T+1)^2 cost matrix per width class) live in shared memory behind
-  // the round masks; when they do not fit the search is left out.  It wants a thread per ordered pair of rounds.
+  // the round masks when they fit (up to about 80 rounds), else in the search's global scratch, which holds a copy of
+  // the same layout (rerank.cuh, rr_carve).  It wants a thread per ordered pair of rounds.
   PlaceLaunch L2 = L;
+  L2.rr_hot_smem = 0;
   if (L2.rr_items && L2.rr_iters > 0) {
-    const size_t N = (size_t)L.prm_T + 1;
-    const size_t need = (size_t)L.J * 8 + RR_MAXCLS * N * N * 8 + 16;
-    int stat = 0;
-    { cudaFuncAttributes fa; if (cudaFuncGetAttributes(&fa, place_kernel<1>) == cudaSuccess) stat = (int)fa.sharedSizeBytes; }
-    if (L.J <= SWB_SMEM_JOBS && smem + need + (size_t)stat <= (size_t)SWB_MAX_DYN_SMEM) {
-      smem += need;
+    if (L.J <= SWB_SMEM_JOBS) {
+      const size_t N = (size_t)L.prm_T + 1;
+      const size_t need = (size_t)L.J * 8 + RR_MAXCLS * N * N * 8 + 16;
+      int stat = 0;
+      { cudaFuncAttributes fa; if (cudaFuncGetAttributes(&fa, place_kernel<1>) == cudaSuccess) stat = (int)fa.sharedSizeBytes; }
+      if (smem + need + (size_t)stat <= (size_t)SWB_MAX_DYN_SMEM) { smem += need; L2.rr_hot_smem = 1; }
       if (nt < 512) nt = 512;
     } else {
       L2.rr_items = nullptr; L2.rr_iters = 0;

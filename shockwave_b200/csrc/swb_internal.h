@@ -60,6 +60,7 @@ struct PlaceLaunch {
   int rr_restarts;        // perturb-and-continue rounds after the first local optimum (iterated local search)
   int prm_T;              // future_rounds of the call (host copy, for sizing)
   int rr_cluster;         // 8: rr_items holds 8 regions per scenario (multi-start over a thread-block cluster), else 1
+  int rr_hot_smem;        // 1: the search's hot arrays (w_j, dense edge costs) sit in shared memory, 0: in rr_items
 };
 
 cudaError_t launch_solve(const SolveLaunch &L, cudaStream_t st, int nbases);

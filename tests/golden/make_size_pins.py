@@ -6,6 +6,9 @@ Run here (no GPU, no reference needed; HiGHS through scipy):
     python tests/golden/make_size_pins.py d-milp   # ~10 min  : the MILP itself at config D with a 900 s limit (HiGHS needs
                                                    #            ~140 s per instance on one core; the reference's 15 s limit
                                                    #            yields no incumbent) -> config_d_milp.json
+    python tests/golden/make_size_pins.py e        # ~18 min  : LP relaxation above 4096 jobs / 64 rounds -> limits_lp.json
+                                                   #            (6144x768x64: 384 s, 8192x1024x32: 158 s, 5000x512x128:
+                                                   #            498 s, one core each)
 Inputs are tests/synth.py instances addressed by (J, G, T, seed, tight); the records keep those keys, the oracle's verdict
 and objective and the seconds it took, so tests/test_gpu_solve.py can rebuild the instance and compare."""
 import json
@@ -26,6 +29,8 @@ D, LAM = 120.0, 12.0
 
 CONFIG_C = [(1024, 128, 32, 1e-3, 1.0, 900), (1024, 128, 20, 1e-3, 3.0, 901), (1024, 128, 32, 1e1, 0.5, 902)]
 CONFIG_D = [(4096, 512, 64, 1e-3, 3.0, 1000), (4096, 512, 64, 1e1, 3.0, 1001), (4096, 512, 64, 1e-3, 0.5, 1002)]
+# the solve's global-memory path (J > 4096) and the high word of the 128-bit round masks (T > 64)
+LIMITS = [(6144, 768, 64, 1e-3, 3.0, 1100), (8192, 1024, 32, 1e1, 3.0, 1101), (5000, 512, 128, 1e-3, 0.5, 1102)]
 
 
 def milp(J, G, T, k, tight, seed, gap, limit):
@@ -63,6 +68,9 @@ if __name__ == "__main__":
     elif what == "d":
         recs = [lp(*p) for p in CONFIG_D]
         path = "config_d_lp.json"
+    elif what == "e":
+        recs = [lp(*p) for p in LIMITS]
+        path = "limits_lp.json"
     else:
         recs = [milp(*p, gap=1e-3, limit=900.0) for p in CONFIG_D[:1]]
         path = "config_d_milp.json"

@@ -53,7 +53,8 @@ def _waterfill(remn, g, G, Tw, tie):
 
 
 def place(n, g, G, T, bfkey, fallback=False, w=None):
-    """Returns dict(x[J][T] bool, backfill[J][T] bool, shortfall, swept_rounds, idle[T])."""
+    """Returns dict(x[J][T] bool, backfill[J][T] bool, shortfall, swept_rounds, sweep_stop, idle[T]); sweep_stop is the
+    round the fallback sweep stopped at, swept_rounds what is left of it after the back-off."""
     n = np.asarray(n, dtype=np.int64)
     g = np.asarray(g, dtype=np.int64)
     J = len(n)
@@ -167,7 +168,7 @@ def place(n, g, G, T, bfkey, fallback=False, w=None):
             if not x[j, t] and g[j] <= room:
                 bf[j, t] = True
                 room -= int(g[j])
-    return dict(x=x, backfill=bf, shortfall=shortfall, swept_rounds=t0, idle=idle)
+    return dict(x=x, backfill=bf, shortfall=shortfall, swept_rounds=t0, sweep_stop=t0_sweep, idle=idle)
 
 
 def _lane_sum(vals, lane):

@@ -111,3 +111,32 @@ def test_schedules_from_matrices_order():
     bf = np.array([[0, 0], [1, 1], [0, 0], [1, 1]], dtype=np.uint8)
     s = schedules_from_matrices(x, bf, np.array([5.0, 9.0, 1.0, 9.0]), [10, 11, 12, 13], 7)
     assert s[7] == [10, 11, 13] and s[8] == [12, 11, 13]
+
+
+@pytest.mark.parametrize("T", [1, 63, 64, 65, 127, 128])
+def test_128_bit_mask_decoders(T):
+    """engine.unpack_masks and the packed form of LazySchedules against the byte matrices, on both words of the mask"""
+    from shockwave_b200.scheduler import LazySchedules
+    rng = np.random.default_rng(T)
+    J = 70
+    x = (rng.random((J, T)) < 0.4).astype(np.uint8)
+    bf = ((rng.random((J, T)) < 0.3) & (x == 0)).astype(np.uint8)
+
+    def pack(m):
+        full = np.zeros((J, 128), dtype=np.uint8)
+        full[:, :T] = m
+        w = (full.reshape(J, 2, 64).astype(np.uint64) << np.arange(64, dtype=np.uint64)).sum(axis=2, dtype=np.uint64)
+        return np.ascontiguousarray(w)
+
+    xm, bm = pack(x), pack(bf)
+    assert np.array_equal(engine.unpack_masks(xm, T), x) and np.array_equal(engine.unpack_masks(bm, T), bf)
+    assert np.array_equal(engine.unpack_masks(xm[None], T), x[None])
+    if T > 64:
+        assert xm[:, 1].any()
+    bfkey = np.round(rng.uniform(0, 50, J))               # ties: the back-fill order must stay stable
+    jobids = list(rng.permutation(1000)[:J])
+    want = schedules_from_matrices(x, bf, bfkey, jobids, 17)
+    got = LazySchedules(None, None, bfkey, jobids, 17, xmask=xm, bfmask=bm, T=T)
+    assert list(got.keys()) == list(want.keys()) == list(range(17, 17 + T))
+    for r in range(17, 17 + T):
+        assert got[r] == want[r], r
