@@ -1,55 +1,14 @@
 // api.cu — the C-ABI of libswb200.so (see include/swb200.h) and the device-memory bookkeeping.
 #include <math.h>
-#include <stdio.h>
 #include <string.h>
 
 #include <string>
 #include <vector>
 
 #include "swb_internal.h"
-#define MK_CHECK_Q(T) (((T) / 4) > 256)
-
-namespace swb {
-cudaError_t launch_place(const PlaceLaunch &L, cudaStream_t st, unsigned long long *gmask);
-}
 
 static thread_local std::string g_err;
 static int fail(int code, const std::string &msg) { g_err = msg; return code; }
-#define CK(call)                                                                            \
-  do {                                                                                      \
-    cudaError_t e_ = (call);                                                                \
-    if (e_ != cudaSuccess)                                                                  \
-      return fail(SWB_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_));        \
-  } while (0)
-
-// growable device buffer
-struct DBuf {
-  void *p = nullptr;
-  size_t cap = 0;
-  cudaError_t need(size_t bytes, cudaStream_t st, bool keep = false) {
-    if (bytes <= cap) return cudaSuccess;
-    size_t ncap = cap ? cap : 256;
-    while (ncap < bytes) ncap *= 2;
-    void *np = nullptr;
-    cudaError_t e = cudaMalloc(&np, ncap);
-    if (e != cudaSuccess) return e;
-    if (keep && p && cap) {
-      e = cudaMemcpyAsync(np, p, cap, cudaMemcpyDeviceToDevice, st);
-      if (e != cudaSuccess) return e;
-      e = cudaStreamSynchronize(st);
-      if (e != cudaSuccess) return e;
-    }
-    if (keep && ncap > cap) {
-      e = cudaMemsetAsync((char *)np + cap, 0, ncap - cap, st);
-      if (e != cudaSuccess) return e;
-    }
-    if (p) cudaFree(p);
-    p = np; cap = ncap;
-    return cudaSuccess;
-  }
-  template <class T> T *as() { return reinterpret_cast<T *>(p); }
-  void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
-};
 
 struct swb_ctx {
   int device = 0;
@@ -80,7 +39,7 @@ struct swb_ctx {
   std::vector<int64_t> h_off;
   std::vector<int32_t> h_E;
   // ---- per-call forecast buffers
-  DBuf f_slots, f_prog, f_mend, f_mns, f_remfb, f_bffb, f_ampok, f_ampfb, f_ftest, f_ncal;
+  DBuf f_remfb, f_bffb, f_ampok, f_ampfb, f_ftest, f_ncal;
   swb::ForecastLaunch last_fc;   // descriptor of the latest forecast (for the calibration commit)
   bool have_fc = false;
   DBuf lp_colp, lp_rowi, lp_val, lp_c, lp_b, lp_Binv, lp_Bm, lp_vec, lp_basis, lp_where, lp_x, lp_out;   // swb_lp_solve
@@ -92,16 +51,12 @@ struct swb_ctx {
   DBuf m_rowprev, m_mj, m_om, m_colprev, m_pi, m_Xc, m_cc, m_pws;   // PDHG state; m_cc = the coarse level's column arrays
   static constexpr int MEV = 32;           // event pairs around the last MEV/2 dense passes of swb_market_pgd
   cudaEvent_t mev[MEV] = {};
-  double last_market_ms = 0.0;
   // CUDA events around the two kernels of the latest solve pass (bench.py's roofline)
   cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
   int last_passes = 0;
-  // pinned staging for the scalar results
-  swb_result *h_res = nullptr;
-  unsigned char *h_stage = nullptr;   // pinned staging of the per-call inputs / outputs of swb_round_solve / swb_forecast
-  size_t h_stage_cap = 0;
-  DBuf f_in;                          // device arena of the per-call forecast inputs (one H2D copy)
-  size_t h_res_cap = 0;
+  PinBuf h_res;     // pinned staging for the scalar results
+  PinBuf h_stage;   // pinned staging of the per-call inputs / outputs of swb_round_solve / swb_forecast
+  DBuf f_in;        // device arena of the per-call forecast inputs (one H2D copy)
 };
 
 extern "C" {
@@ -138,26 +93,10 @@ int swb_create(swb_ctx **out, int device) {
 void swb_destroy(swb_ctx *c) {
   if (!c) return;
   cudaSetDevice(c->device);
-  DBuf *all[] = {&c->prm, &c->res, &c->g, &c->E, &c->c, &c->dbar, &c->rem, &c->ftobj, &c->bfkey, &c->x,
-                 &c->bf, &c->nr, &c->w, &c->xmk, &c->bmk, &c->sa, &c->su0, &c->sR, &c->sws, &c->scap, &c->sg, &c->snF,
-                 &c->snmax, &c->sn, &c->gmask, &c->sncap, &c->seated, &c->scth, &c->sRr, &c->sths, &c->sn0, &c->snfc, &c->t_off, &c->t_E, &c->t_nm, &c->t_g, &c->t_ns, &c->t_ts,
-                 &c->t_modes, &c->t_mm, &c->t_amp, &c->s_r0, &c->s_rl, &c->s_cnt, &c->s_vl, &c->s_acc, &c->t_mu, &c->t_sg, &c->ens_z, &c->gv_in, &c->gv_out, &c->rr_items,
-                 &c->pool_pp, &c->pool_bs, &c->f_slots, &c->f_prog, &c->f_mend, &c->f_mns, &c->f_remfb,
-                 &c->f_bffb, &c->f_ampok, &c->f_ampfb, &c->f_ftest, &c->f_ncal, &c->lp_colp, &c->lp_rowi, &c->lp_val, &c->lp_c, &c->lp_b, &c->lp_Binv, &c->lp_Bm, &c->lp_vec, &c->lp_basis, &c->lp_where, &c->lp_x, &c->lp_out, &c->ax_p, &c->ax_t, &c->ax_wt, &c->ax_u, &c->ax_v, &c->ax_spc, &c->ax_c4r, &c->ax_r4c,
-                 &c->ax_path, &c->ax_sc, &c->ax_sr, &c->ax_out, &c->pol_coef, &c->pol_sf, &c->pol_t,
-                 &c->pol_n, &c->pol_den, &c->pol_x, &c->pol_out, &c->mc_R0, &c->mc_mu, &c->mc_sigma, &c->mc_H, &c->mc_out,
-                 &c->m_theta, &c->m_rowp, &c->m_colload,
-                 &c->m_colscale, &c->m_price, &c->m_obj, &c->m_X, &c->m_rate, &c->m_E, &c->m_c, &c->m_Gw,
-                 &c->m_rowprev, &c->m_mj, &c->m_om, &c->m_colprev, &c->m_pi, &c->m_Xc, &c->m_cc, &c->m_pws,
-                 &c->het_a, &c->het_N, &c->het_x, &c->wf_z, &c->wf_x2};
-  for (DBuf *b : all) b->release();
-  if (c->h_res) cudaFreeHost(c->h_res);
-  if (c->h_stage) cudaFreeHost(c->h_stage);
-  c->f_in.release();
   for (int i = 0; i < 3; ++i) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
   for (int i = 0; i < swb_ctx::MEV; ++i) if (c->mev[i]) cudaEventDestroy(c->mev[i]);
   if (c->st) cudaStreamDestroy(c->st);
-  delete c;
+  delete c;      // the buffers free themselves
 }
 
 void *swb_stream(swb_ctx *c) { return c ? (void *)c->st : nullptr; }
@@ -190,28 +129,6 @@ static int ensure_scratch(swb_ctx *c, size_t n) {
   return 0;
 }
 
-static int ensure_hres(swb_ctx *c, size_t S) {
-  if (S > c->h_res_cap) {
-    if (c->h_res) cudaFreeHost(c->h_res);
-    c->h_res = nullptr;
-    CK(cudaMallocHost((void **)&c->h_res, S * sizeof(swb_result)));
-    c->h_res_cap = S;
-  }
-  return 0;
-}
-
-static int ensure_hstage(swb_ctx *c, size_t bytes) {
-  if (bytes > c->h_stage_cap) {
-    if (c->h_stage) cudaFreeHost(c->h_stage);
-    c->h_stage = nullptr; c->h_stage_cap = 0;
-    size_t cap = 1 << 16;
-    while (cap < bytes) cap *= 2;
-    CK(cudaMallocHost((void **)&c->h_stage, cap));
-    c->h_stage_cap = cap;
-  }
-  return 0;
-}
-
 // common tail: launch solve + place on device-resident inputs
 static int run_solve(swb_ctx *c, int S, int J, int per_scn, const swb_params *h_prm, const int32_t *g,
                      const int32_t *E, const int32_t *cc, const double *dbar, const double *rem,
@@ -222,9 +139,8 @@ static int run_solve(swb_ctx *c, int S, int J, int per_scn, const swb_params *h_
   const size_t n = (size_t)S * J;
   int rc = ensure_scratch(c, n);
   if (rc) return rc;
-  CK(c->prm.need(sizeof(swb_params) * S, c->st));
   CK(c->res.need(sizeof(swb_result) * S, c->st));
-  CK(cudaMemcpyAsync(c->prm.p, h_prm, sizeof(swb_params) * S, cudaMemcpyHostToDevice, c->st));
+  CK(c->prm.upload(h_prm, sizeof(swb_params) * S, c->st));
   if (J > SWB_SMEM_JOBS) {
     CK(c->gmask.need(n * 4 * sizeof(unsigned long long), c->st));
     CK(c->scth.need(n * 8, c->st)); CK(c->sRr.need(n * 8, c->st)); CK(c->sths.need(n * SWB_MAX_BASES * 4, c->st));
@@ -264,8 +180,8 @@ static int run_solve(swb_ctx *c, int S, int J, int per_scn, const swb_params *h_
       P.rr_items = c->rr_items.p; P.rr_iters = c->rr_iters; P.rr_restarts = c->rr_restarts; P.rr_cluster = cl;
     }
   }
-  int rc2 = ensure_hres(c, S);
-  if (rc2) return rc2;
+  CK(c->h_res.need(sizeof(swb_result) * S));
+  const swb_result *hres = c->h_res.as<swb_result>();
   for (int pass = 0; pass < SWB_MAX_REPLAN + 1; ++pass) {
     CK(cudaEventRecord(c->ev[0], c->st));
     CK(swb::launch_solve(L, c->st, h_prm[0].nbases));
@@ -273,10 +189,10 @@ static int run_solve(swb_ctx *c, int S, int J, int per_scn, const swb_params *h_
     CK(swb::launch_place(P, c->st, c->gmask.as<unsigned long long>()));
     CK(cudaEventRecord(c->ev[2], c->st));
     c->last_passes = pass + 1;
-    CK(cudaMemcpyAsync(c->h_res, c->res.p, sizeof(swb_result) * S, cudaMemcpyDeviceToHost, c->st));
+    CK(cudaMemcpyAsync(c->h_res.p, c->res.p, sizeof(swb_result) * S, cudaMemcpyDeviceToHost, c->st));
     CK(cudaStreamSynchronize(c->st));
     int shortf = 0;
-    for (int s = 0; s < S; ++s) shortf += c->h_res[s].shortfall;
+    for (int s = 0; s < S; ++s) shortf += hres[s].shortfall;
     if (shortf == 0 || pass == SWB_MAX_REPLAN) break;
     // place_kernel has already written the tighter per-job caps for the next pass (packing feedback)
   }
@@ -315,16 +231,13 @@ int swb_solve(swb_ctx *c, const swb_solve_args *a) {
     bfkey = a->bfkey ? a->bfkey : a->rem;
     x = a->x; bf = a->backfill; nr = a->nrounds; w = a->weights;
   } else {
-    CK(c->g.need(nj * 4, c->st)); CK(c->E.need(nj * 4, c->st)); CK(c->c.need(nj * 4, c->st));
-    CK(c->dbar.need(nj * 8, c->st)); CK(c->rem.need(nj * 8, c->st)); CK(c->ftobj.need(nj * 8, c->st));
-    CK(c->bfkey.need(nj * 8, c->st));
-    CK(cudaMemcpyAsync(c->g.p, a->g, nj * 4, cudaMemcpyHostToDevice, c->st));
-    CK(cudaMemcpyAsync(c->E.p, a->E, nj * 4, cudaMemcpyHostToDevice, c->st));
-    CK(cudaMemcpyAsync(c->c.p, a->c, nj * 4, cudaMemcpyHostToDevice, c->st));
-    CK(cudaMemcpyAsync(c->dbar.p, a->dbar, nj * 8, cudaMemcpyHostToDevice, c->st));
-    CK(cudaMemcpyAsync(c->rem.p, a->rem, nj * 8, cudaMemcpyHostToDevice, c->st));
-    CK(cudaMemcpyAsync(c->ftobj.p, a->ftobj, nj * 8, cudaMemcpyHostToDevice, c->st));
-    CK(cudaMemcpyAsync(c->bfkey.p, a->bfkey ? a->bfkey : a->rem, nj * 8, cudaMemcpyHostToDevice, c->st));
+    CK(c->g.upload(a->g, nj * 4, c->st));
+    CK(c->E.upload(a->E, nj * 4, c->st));
+    CK(c->c.upload(a->c, nj * 4, c->st));
+    CK(c->dbar.upload(a->dbar, nj * 8, c->st));
+    CK(c->rem.upload(a->rem, nj * 8, c->st));
+    CK(c->ftobj.upload(a->ftobj, nj * 8, c->st));
+    CK(c->bfkey.upload(a->bfkey ? a->bfkey : a->rem, nj * 8, c->st));
     g = c->g.as<int32_t>(); E = c->E.as<int32_t>(); cc = c->c.as<int32_t>();
     dbar = c->dbar.as<double>(); rem = c->rem.as<double>(); ftobj = c->ftobj.as<double>();
     bfkey = c->bfkey.as<double>();
@@ -338,9 +251,7 @@ int swb_solve(swb_ctx *c, const swb_solve_args *a) {
   rc = run_solve(c, S, J, a->per_scenario_jobs, a->prm, g, E, cc, dbar, rem, ftobj, bfkey, nullptr,
                  nullptr, x, bf, nr, w, nullptr, xmk, bmk);
   if (rc) return rc;
-  rc = ensure_hres(c, S);
-  if (rc) return rc;
-  CK(cudaMemcpyAsync(c->h_res, c->res.p, sizeof(swb_result) * S, cudaMemcpyDeviceToHost, c->st));
+  CK(cudaMemcpyAsync(c->h_res.p, c->res.p, sizeof(swb_result) * S, cudaMemcpyDeviceToHost, c->st));
   if (!a->on_device) {
     if (a->x) CK(cudaMemcpyAsync(a->x, x, nx, cudaMemcpyDeviceToHost, c->st));
     if (a->backfill) CK(cudaMemcpyAsync(a->backfill, bf, nx, cudaMemcpyDeviceToHost, c->st));
@@ -351,7 +262,7 @@ int swb_solve(swb_ctx *c, const swb_solve_args *a) {
     if (a->bfmask) CK(cudaMemcpyAsync(a->bfmask, bmk, (size_t)S * J * 16, cudaMemcpyDeviceToHost, c->st));
   }
   CK(cudaStreamSynchronize(c->st));
-  memcpy(a->res, c->h_res, sizeof(swb_result) * S);
+  memcpy(a->res, c->h_res.p, sizeof(swb_result) * S);
   for (int s = 0; s < S; ++s)
     if (a->res[s].flags & 1) return fail(SWB_ERR_ARG, "swb_solve: gang width g[j] must be in [1, 255] (device input)");
   int any_fb = 0;
@@ -573,13 +484,13 @@ static int run_forecast(swb_ctx *c, const swb_params *prm, const swb_round_args 
   // pageable memory is a staged, synchronous copy of its own (every API call ends with a stream sync, so the staging
   // buffer is free again when the next call starts)
   const size_t Jz = (size_t)J;
-  { int rcs = ensure_hstage(c, 84 * Jz + 64); if (rcs) return rcs; }
-  CK(c->f_in.need(20 * Jz, c->st));
-  memcpy(c->h_stage, a->meas_nsamples, 8 * Jz);
-  memcpy(c->h_stage + 8 * Jz, a->slots, 4 * Jz);
-  memcpy(c->h_stage + 12 * Jz, a->epoch_progress, 4 * Jz);
-  memcpy(c->h_stage + 16 * Jz, a->meas_end_round, 4 * Jz);
-  CK(cudaMemcpyAsync(c->f_in.p, c->h_stage, 20 * Jz, cudaMemcpyHostToDevice, c->st));
+  CK(c->h_stage.need(84 * Jz + 64));
+  unsigned char *hs = c->h_stage.as<unsigned char>();
+  memcpy(hs, a->meas_nsamples, 8 * Jz);
+  memcpy(hs + 8 * Jz, a->slots, 4 * Jz);
+  memcpy(hs + 12 * Jz, a->epoch_progress, 4 * Jz);
+  memcpy(hs + 16 * Jz, a->meas_end_round, 4 * Jz);
+  CK(c->f_in.upload(hs, 20 * Jz, c->st));
   unsigned char *din = reinterpret_cast<unsigned char *>(c->f_in.p);
   swb::ForecastLaunch F;
   F.J = J; F.reestimate_share = a->reestimate_share; F.round_ptr = prm->round_ptr; F.ngpus = prm->ngpus;
@@ -646,14 +557,12 @@ int swb_round_solve(swb_ctx *c, const swb_params *prm, const swb_round_args *a) 
                  c->nr.as<int32_t>(), nullptr, c->f_ncal.as<int32_t>(), dxm, dbm);
   if (rc) return rc;
   CK(swb::launch_commit_calibration(c->last_fc, c->res.as<swb_result>(), 0, c->f_ncal.as<int32_t>(), c->st));
-  rc = ensure_hres(c, 1);
-  if (rc) return rc;
-  CK(cudaMemcpyAsync(c->h_res, c->res.p, sizeof(swb_result), cudaMemcpyDeviceToHost, c->st));
+  CK(cudaMemcpyAsync(c->h_res.p, c->res.p, sizeof(swb_result), cudaMemcpyDeviceToHost, c->st));
   if (a->x) CK(cudaMemcpyAsync(a->x, c->x.p, nx, cudaMemcpyDeviceToHost, c->st));
   if (a->backfill) CK(cudaMemcpyAsync(a->backfill, c->bf.p, nx, cudaMemcpyDeviceToHost, c->st));
   // the packed outputs (84 bytes per job) come back through the pinned staging buffer — truly asynchronous copies and
   // one sync — and are handed to the caller's (pageable) arrays by memcpy
-  unsigned char *hs = c->h_stage;
+  unsigned char *hs = c->h_stage.as<unsigned char>();
   const size_t Jz = (size_t)J;
   if (a->xmask) CK(cudaMemcpyAsync(hs, dxm, 16 * Jz, cudaMemcpyDeviceToHost, c->st));
   if (a->bfmask) CK(cudaMemcpyAsync(hs + 16 * Jz, dbm, 16 * Jz, cudaMemcpyDeviceToHost, c->st));
@@ -672,7 +581,7 @@ int swb_round_solve(swb_ctx *c, const swb_params *prm, const swb_round_args *a) 
   if (a->bfmask) memcpy(a->bfmask, hs + 16 * Jz, 16 * Jz);
   if (a->nrounds) memcpy(a->nrounds, hs + 32 * Jz, 4 * Jz);
   if (a->forecast_out) memcpy(a->forecast_out, hs + 36 * Jz, 48 * Jz);
-  *a->res = *c->h_res;
+  *a->res = *c->h_res.as<swb_result>();
   return a->res->status == SWB_ST_FALLBACK ? SWB_ST_FALLBACK : SWB_ST_OK;
 }
 
@@ -703,11 +612,10 @@ int swb_policy_pooled(swb_ctx *c, int32_t mode, int32_t J, double N, const doubl
   if (mode == SWB_POL_MTD && !n) return fail(SWB_ERR_ARG, "swb_policy_pooled: MTD needs n");
   CK(cudaSetDevice(c->device));
   const size_t b = (size_t)J * 8;
-  CK(c->pol_coef.need(b, c->st)); CK(c->pol_sf.need(b, c->st)); CK(c->pol_t.need(b, c->st));
-  CK(c->pol_n.need(b, c->st)); CK(c->pol_den.need(b, c->st)); CK(c->pol_x.need(b, c->st));
-  CK(c->pol_out.need(16, c->st));
-  CK(cudaMemcpyAsync(c->pol_coef.p, coef, b, cudaMemcpyHostToDevice, c->st));
-  CK(cudaMemcpyAsync(c->pol_sf.p, sf, b, cudaMemcpyHostToDevice, c->st));
+  CK(c->pol_t.need(b, c->st)); CK(c->pol_n.need(b, c->st)); CK(c->pol_den.need(b, c->st));
+  CK(c->pol_x.need(b, c->st)); CK(c->pol_out.need(16, c->st));
+  CK(c->pol_coef.upload(coef, b, c->st));
+  CK(c->pol_sf.upload(sf, b, c->st));
   if (t) CK(cudaMemcpyAsync(c->pol_t.p, t, b, cudaMemcpyHostToDevice, c->st));
   if (n) CK(cudaMemcpyAsync(c->pol_n.p, n, b, cudaMemcpyHostToDevice, c->st));
   if (den) CK(cudaMemcpyAsync(c->pol_den.p, den, b, cudaMemcpyHostToDevice, c->st));
@@ -740,13 +648,12 @@ int swb_policy_hetero(swb_ctx *c, int32_t mode, int32_t J, int32_t W, const doub
     if (!(N[w] > 0.0)) return fail(SWB_ERR_ARG, "swb_policy_hetero: every worker type needs capacity > 0 (drop empty types)");
   CK(cudaSetDevice(c->device));
   const size_t b = (size_t)J * 8, bw = b * (size_t)W;
-  CK(c->het_a.need(bw, c->st)); CK(c->het_x.need(bw, c->st)); CK(c->het_N.need(32, c->st));
-  CK(c->pol_sf.need(b, c->st)); CK(c->pol_t.need(b, c->st));
-  CK(c->pol_n.need(b, c->st)); CK(c->pol_den.need(b, c->st));
+  CK(c->het_x.need(bw, c->st)); CK(c->het_N.need(32, c->st));
+  CK(c->pol_t.need(b, c->st)); CK(c->pol_n.need(b, c->st)); CK(c->pol_den.need(b, c->st));
   CK(c->pol_out.need(128, c->st));
-  CK(cudaMemcpyAsync(c->het_a.p, a, bw, cudaMemcpyHostToDevice, c->st));
+  CK(c->het_a.upload(a, bw, c->st));
   CK(cudaMemcpyAsync(c->het_N.p, N, (size_t)W * 8, cudaMemcpyHostToDevice, c->st));
-  CK(cudaMemcpyAsync(c->pol_sf.p, sf, b, cudaMemcpyHostToDevice, c->st));
+  CK(c->pol_sf.upload(sf, b, c->st));
   if (t) CK(cudaMemcpyAsync(c->pol_t.p, t, b, cudaMemcpyHostToDevice, c->st));
   if (n) CK(cudaMemcpyAsync(c->pol_n.p, n, b, cudaMemcpyHostToDevice, c->st));
   // MAXSUM with SLO floors: t = needed throughput per job, den = instance cost per worker type (W entries)
@@ -766,11 +673,6 @@ int swb_policy_hetero(swb_ctx *c, int32_t mode, int32_t J, int32_t W, const doub
   CK(cudaStreamSynchronize(c->st));
   if (objective) *objective = out[0];
   if (stats) { stats[0] = (int32_t)out[2]; stats[1] = (int32_t)out[3]; }
-  if (getenv("SWB_HETERO_DEBUG")) {
-    fprintf(stderr, "hetero dbg:");
-    for (int i = 4; i < 16; ++i) fprintf(stderr, " %.17g", out[i]);
-    fprintf(stderr, "\n");
-  }
   return out[1] != 0.0 ? 1 : 0;
 }
 
@@ -789,16 +691,14 @@ int swb_policy_waterfill_step(swb_ctx *c, int32_t J, int32_t W, const double *N,
       return fail(SWB_ERR_ARG, "swb_policy_waterfill_step: prop and sf must be positive, mult non-negative");
   CK(cudaSetDevice(c->device));
   const size_t b = (size_t)J * 8, bw = b * (size_t)W;
-  CK(c->het_a.need(bw, c->st)); CK(c->het_x.need(bw, c->st)); CK(c->het_N.need(32, c->st));
-  CK(c->pol_sf.need(b, c->st)); CK(c->pol_t.need(b, c->st));
-  CK(c->pol_n.need(b, c->st)); CK(c->pol_den.need(b, c->st));
+  CK(c->het_x.need(bw, c->st)); CK(c->het_N.need(32, c->st));
   CK(c->pol_out.need(256, c->st)); CK(c->wf_z.need(b, c->st)); CK(c->wf_x2.need(bw, c->st));
-  CK(cudaMemcpyAsync(c->het_a.p, thr, bw, cudaMemcpyHostToDevice, c->st));
+  CK(c->het_a.upload(thr, bw, c->st));
   CK(cudaMemcpyAsync(c->het_N.p, N, (size_t)W * 8, cudaMemcpyHostToDevice, c->st));
-  CK(cudaMemcpyAsync(c->pol_sf.p, sf, b, cudaMemcpyHostToDevice, c->st));
-  CK(cudaMemcpyAsync(c->pol_t.p, lower, b, cudaMemcpyHostToDevice, c->st));
-  CK(cudaMemcpyAsync(c->pol_n.p, mult, b, cudaMemcpyHostToDevice, c->st));
-  CK(cudaMemcpyAsync(c->pol_den.p, prop, b, cudaMemcpyHostToDevice, c->st));
+  CK(c->pol_sf.upload(sf, b, c->st));
+  CK(c->pol_t.upload(lower, b, c->st));
+  CK(c->pol_n.upload(mult, b, c->st));
+  CK(c->pol_den.upload(prop, b, c->st));
   swb::HeteroLaunch L;
   L.mode = SWB_POL_WFILL; L.J = J; L.W = W;
   L.N = c->het_N.as<double>(); L.a = c->het_a.as<double>(); L.sf = c->pol_sf.as<double>();
@@ -839,12 +739,10 @@ int swb_gbm_forecast(swb_ctx *c, int32_t J, const double *R0, const int32_t *H, 
   if (in_dev) {
     L.R0 = R0; L.mu = mu; L.sigma = sigma; L.H = H;
   } else {
-    CK(c->mc_R0.need(b, c->st)); CK(c->mc_mu.need(b, c->st)); CK(c->mc_sigma.need(b, c->st));
-    CK(c->mc_H.need((size_t)J * 4, c->st));
-    CK(cudaMemcpyAsync(c->mc_R0.p, R0, b, cudaMemcpyHostToDevice, c->st));
-    CK(cudaMemcpyAsync(c->mc_mu.p, mu, b, cudaMemcpyHostToDevice, c->st));
-    CK(cudaMemcpyAsync(c->mc_sigma.p, sigma, b, cudaMemcpyHostToDevice, c->st));
-    CK(cudaMemcpyAsync(c->mc_H.p, H, (size_t)J * 4, cudaMemcpyHostToDevice, c->st));
+    CK(c->mc_R0.upload(R0, b, c->st));
+    CK(c->mc_mu.upload(mu, b, c->st));
+    CK(c->mc_sigma.upload(sigma, b, c->st));
+    CK(c->mc_H.upload(H, (size_t)J * 4, c->st));
     L.R0 = c->mc_R0.as<double>(); L.mu = c->mc_mu.as<double>(); L.sigma = c->mc_sigma.as<double>();
     L.H = c->mc_H.as<int32_t>();
   }
@@ -897,8 +795,8 @@ int swb_gavel_round(swb_ctx *c, const swb_gavel_round_args *a) {
   const size_t o_order = put(a->type_order, W), o_cap = put(a->capacity, W), o_sf = put(a->sf, J),
                o_nw = put(a->nworkers, W), o_wid = put(a->worker_ids, totw), o_pt = put(a->prev_type, J),
                o_po = put(a->prev_off, J + 1), o_pl = put(a->prev_local, nprev);
-  CK(c->gv_in.need(in_bytes, c->st)); CK(c->gv_out.need(out_bytes, c->st));
-  CK(cudaMemcpyAsync(c->gv_in.p, h.data(), in_bytes, cudaMemcpyHostToDevice, c->st));
+  CK(c->gv_out.need(out_bytes, c->st));
+  CK(c->gv_in.upload(h.data(), in_bytes, c->st));
   const double *dd = c->gv_in.as<double>();
   const int32_t *di = reinterpret_cast<const int32_t *>(dd + nd_in);
   double *od = c->gv_out.as<double>();
@@ -945,8 +843,7 @@ int swb_gbm_ensemble(swb_ctx *c, int32_t S, int32_t J, double P_total, const dou
   if (!c || !sums_dev || !z || !rem_out_dev) return fail(SWB_ERR_ARG, "swb_gbm_ensemble: null argument");
   if (S <= 0 || J <= 0 || !(P_total > 0.0)) return fail(SWB_ERR_ARG, "swb_gbm_ensemble: bad S / J / P_total");
   CK(cudaSetDevice(c->device));
-  CK(c->ens_z.need((size_t)S * 8, c->st));
-  CK(cudaMemcpyAsync(c->ens_z.p, z, (size_t)S * 8, cudaMemcpyHostToDevice, c->st));
+  CK(c->ens_z.upload(z, (size_t)S * 8, c->st));
   CK(swb::launch_gbm_ensemble(S, J, P_total, sums_dev, c->ens_z.as<double>(), rem_out_dev, c->st));
   if (!c->aux_async) CK(cudaStreamSynchronize(c->st));
   return 0;
@@ -982,7 +879,6 @@ int swb_market_pgd(swb_ctx *c, const swb_market_args *a) {
   const int S = a->S, J = a->J, W = a->W, T = a->T;
   if (S <= 0 || J <= 0 || W <= 0 || W > SWB_MK_MAXW || T <= 0 || (T & 3) || T > 1024)
     return fail(SWB_ERR_ARG, "swb_market_pgd: need W in [1,4], T a multiple of 4, T <= 1024");
-  if (MK_CHECK_Q(T)) return fail(SWB_ERR_ARG, "swb_market_pgd: T/4 must not exceed 256");
   if (a->iters < 0 || a->coarse_iters < 0 || a->primal_weight < 0.f)
     return fail(SWB_ERR_ARG, "swb_market_pgd: negative iteration count or primal weight");
   const int TC = 4, grp = T / TC;
@@ -1004,14 +900,13 @@ int swb_market_pgd(swb_ctx *c, const swb_market_args *a) {
   CK(cudaSetDevice(c->device));
   const size_t nj = a->per_scenario_jobs ? (size_t)S * J : (size_t)J, sj = (size_t)S * J;
   const size_t nx = sj * W * T, nwt = (size_t)S * W * T, nwc = (size_t)S * W * TC;
-  CK(c->prm.need(sizeof(swb_params) * S, c->st));
-  CK(cudaMemcpyAsync(c->prm.p, a->prm, sizeof(swb_params) * S, cudaMemcpyHostToDevice, c->st));
+  CK(c->prm.upload(a->prm, sizeof(swb_params) * S, c->st));
   CK(c->m_theta.need(sj * 16, c->st)); CK(c->m_rowp.need(sj * 4, c->st));
   CK(c->m_rowprev.need(sj * 4, c->st)); CK(c->m_mj.need(sj * 8, c->st)); CK(c->m_om.need(sj * 8, c->st));
   CK(c->m_colload.need(nwt * 4, c->st)); CK(c->m_colscale.need(nwt * 4, c->st)); CK(c->m_price.need(nwt * 4, c->st));
   CK(c->m_colprev.need(nwt * 4, c->st)); CK(c->m_pi.need(nwt * 8, c->st));
-  CK(c->m_obj.need((size_t)S * 3 * 8, c->st)); CK(c->m_Gw.need(icap.size() * 4, c->st));
-  CK(cudaMemcpyAsync(c->m_Gw.p, icap.data(), icap.size() * 4, cudaMemcpyHostToDevice, c->st));
+  CK(c->m_obj.need((size_t)S * 3 * 8, c->st));
+  CK(c->m_Gw.upload(icap.data(), icap.size() * 4, c->st));
   swb::MarketLaunch L;
   L.S = S; L.J = J; L.W = W; L.T = T; L.per_scn = a->per_scenario_jobs;
   L.Tfull = T; L.rscale = 1.f;
@@ -1019,15 +914,13 @@ int swb_market_pgd(swb_ctx *c, const swb_market_args *a) {
   if (a->on_device) {
     L.g = a->g; L.E = a->E; L.c = a->c; L.dbar = a->dbar; L.rem = a->rem; L.rate = a->rate; L.X = a->X;
   } else {
-    CK(c->g.need(nj * 4, c->st)); CK(c->m_E.need(nj * 8, c->st)); CK(c->m_c.need(nj * 8, c->st));
-    CK(c->dbar.need(nj * 8, c->st)); CK(c->rem.need(nj * 8, c->st)); CK(c->m_rate.need(nj * W * 4, c->st));
+    CK(c->g.upload(a->g, nj * 4, c->st));
+    CK(c->m_E.upload(a->E, nj * 8, c->st));
+    CK(c->m_c.upload(a->c, nj * 8, c->st));
+    CK(c->dbar.upload(a->dbar, nj * 8, c->st));
+    CK(c->rem.upload(a->rem, nj * 8, c->st));
+    CK(c->m_rate.upload(a->rate, nj * W * 4, c->st));
     CK(c->m_X.need(nx * 4, c->st));
-    CK(cudaMemcpyAsync(c->g.p, a->g, nj * 4, cudaMemcpyHostToDevice, c->st));
-    CK(cudaMemcpyAsync(c->m_E.p, a->E, nj * 8, cudaMemcpyHostToDevice, c->st));
-    CK(cudaMemcpyAsync(c->m_c.p, a->c, nj * 8, cudaMemcpyHostToDevice, c->st));
-    CK(cudaMemcpyAsync(c->dbar.p, a->dbar, nj * 8, cudaMemcpyHostToDevice, c->st));
-    CK(cudaMemcpyAsync(c->rem.p, a->rem, nj * 8, cudaMemcpyHostToDevice, c->st));
-    CK(cudaMemcpyAsync(c->m_rate.p, a->rate, nj * W * 4, cudaMemcpyHostToDevice, c->st));
     if (a->warm_start) CK(cudaMemcpyAsync(c->m_X.p, a->X, nx * 4, cudaMemcpyHostToDevice, c->st));
     L.g = c->g.as<int32_t>(); L.E = c->m_E.as<double>(); L.c = c->m_c.as<double>();
     L.dbar = c->dbar.as<double>(); L.rem = c->rem.as<double>(); L.rate = c->m_rate.as<float>();
@@ -1047,8 +940,7 @@ int swb_market_pgd(swb_ctx *c, const swb_market_args *a) {
   CK(c->m_pws.need((size_t)S * 4, c->st));
   L.pws = c->m_pws.as<float>();
   L.phase = 0; L.mode = 0;
-  int split = 8;                       // CTAs per scenario (8 sweeps per thread at 4096 jobs x 64 rounds)
-  if (const char *e = getenv("SWB_MK_SPLIT")) { const int v = atoi(e); if (v > 0) split = v; }
+  const int split = 8;                 // CTAs per scenario (8 sweeps per thread at 4096 jobs x 64 rounds)
   auto tile = [&](int Tl) {            // jobs per CTA: enough CTAs to fill the GPU, long sweeps so the column accumulators pay
     int per = (J + split - 1) / split;
     const int sweep = 256 / (Tl / 4) > 0 ? 256 / (Tl / 4) : 1;
@@ -1100,7 +992,6 @@ int swb_market_pgd(swb_ctx *c, const swb_market_args *a) {
     }
     dense_ms = n ? (float)(acc / n) : 0.f;
   }
-  c->last_market_ms = dense_ms;
   if (a->dense_ms) *a->dense_ms = dense_ms;
   return 0;
 }
@@ -1125,14 +1016,13 @@ int swb_allox_assign(swb_ctx *c, int32_t m, int32_t n, int32_t W, const double *
     return fail(SWB_ERR_ARG, "swb_allox_assign: need m, n > 0 and m*n <= 2^26");
   CK(cudaSetDevice(c->device));
   const size_t N = (size_t)m * n;
-  CK(c->ax_p.need((size_t)m * W * 8, c->st)); CK(c->ax_t.need((size_t)m * 8, c->st));
-  CK(c->ax_wt.need((size_t)n * 4, c->st)); CK(c->ax_u.need((size_t)m * 8, c->st));
+  CK(c->ax_u.need((size_t)m * 8, c->st));
   CK(c->ax_v.need(N * 8, c->st)); CK(c->ax_spc.need(N * 8, c->st));
   CK(c->ax_c4r.need((size_t)m * 4, c->st)); CK(c->ax_r4c.need(N * 4, c->st)); CK(c->ax_path.need(N * 4, c->st));
   CK(c->ax_sc.need(N, c->st)); CK(c->ax_sr.need((size_t)m, c->st)); CK(c->ax_out.need(8, c->st));
-  CK(cudaMemcpyAsync(c->ax_p.p, p, (size_t)m * W * 8, cudaMemcpyHostToDevice, c->st));
-  CK(cudaMemcpyAsync(c->ax_t.p, t, (size_t)m * 8, cudaMemcpyHostToDevice, c->st));
-  CK(cudaMemcpyAsync(c->ax_wt.p, wtype, (size_t)n * 4, cudaMemcpyHostToDevice, c->st));
+  CK(c->ax_p.upload(p, (size_t)m * W * 8, c->st));
+  CK(c->ax_t.upload(t, (size_t)m * 8, c->st));
+  CK(c->ax_wt.upload(wtype, (size_t)n * 4, c->st));
   swb::AssignLaunch L;
   L.m = m; L.n = n; L.W = W;
   L.p = c->ax_p.as<double>(); L.t = c->ax_t.as<double>(); L.wtype = c->ax_wt.as<int32_t>();
@@ -1164,18 +1054,17 @@ int swb_lp_solve(swb_ctx *c, int32_t S, int32_t m, int32_t n, int32_t nnz, const
     if (rowi[k] < 0 || rowi[k] >= m) return fail(SWB_ERR_ARG, "swb_lp_solve: row index out of range");
   CK(cudaSetDevice(c->device));
   const size_t sm = (size_t)S * m, sn = (size_t)S * n, snz = (size_t)S * (nnz > 0 ? nnz : 1);
-  CK(c->lp_colp.need((size_t)(n + 1) * 4, c->st)); CK(c->lp_rowi.need((size_t)(nnz > 0 ? nnz : 1) * 4, c->st));
-  CK(c->lp_val.need(snz * 8, c->st)); CK(c->lp_c.need(sn * 8, c->st)); CK(c->lp_b.need(sm * 8, c->st));
+  CK(c->lp_rowi.need((size_t)(nnz > 0 ? nnz : 1) * 4, c->st)); CK(c->lp_val.need(snz * 8, c->st));
   CK(c->lp_Binv.need(sm * m * 8, c->st)); CK(c->lp_Bm.need(sm * m * 8, c->st)); CK(c->lp_vec.need(sm * 5 * 8, c->st));
   CK(c->lp_basis.need(sm * 4, c->st)); CK(c->lp_where.need((size_t)S * (n + m + 1) * 4, c->st));
   CK(c->lp_x.need(sn * 8, c->st)); CK(c->lp_out.need((size_t)S * 64, c->st));
-  CK(cudaMemcpyAsync(c->lp_colp.p, colp, (size_t)(n + 1) * 4, cudaMemcpyHostToDevice, c->st));
+  CK(c->lp_colp.upload(colp, (size_t)(n + 1) * 4, c->st));
   if (nnz > 0) {
     CK(cudaMemcpyAsync(c->lp_rowi.p, rowi, (size_t)nnz * 4, cudaMemcpyHostToDevice, c->st));
     CK(cudaMemcpyAsync(c->lp_val.p, val, (size_t)S * nnz * 8, cudaMemcpyHostToDevice, c->st));
   }
-  CK(cudaMemcpyAsync(c->lp_c.p, cost, sn * 8, cudaMemcpyHostToDevice, c->st));
-  CK(cudaMemcpyAsync(c->lp_b.p, b, sm * 8, cudaMemcpyHostToDevice, c->st));
+  CK(c->lp_c.upload(cost, sn * 8, c->st));
+  CK(c->lp_b.upload(b, sm * 8, c->st));
   swb::LpLaunch L;
   L.S = S; L.m = m; L.n = n; L.nnz = nnz; L.max_iter = max_iter;
   L.colp = c->lp_colp.as<int>(); L.rowi = c->lp_rowi.as<int>();
@@ -1214,8 +1103,7 @@ int swb_forecast_commit(swb_ctx *c, int32_t J, int32_t fallback, const int32_t *
   if (!c || !ncal) return fail(SWB_ERR_ARG, "swb_forecast_commit: null argument");
   if (!c->have_fc || c->last_fc.J != J) return fail(SWB_ERR_STATE, "swb_forecast_commit: no matching forecast");
   CK(cudaSetDevice(c->device));
-  CK(c->f_ncal.need((size_t)J * 4, c->st));
-  CK(cudaMemcpyAsync(c->f_ncal.p, ncal, (size_t)J * 4, cudaMemcpyHostToDevice, c->st));
+  CK(c->f_ncal.upload(ncal, (size_t)J * 4, c->st));
   CK(swb::launch_commit_calibration(c->last_fc, nullptr, fallback, c->f_ncal.as<int32_t>(), c->st));
   CK(cudaStreamSynchronize(c->st));
   c->have_fc = false;

@@ -46,24 +46,16 @@ struct swb_sim {
   int device = 0, S = 0, J = 0, ngpus = 0, begun = 0;
   double tpi = 0, grd = 0;
   cudaStream_t st = nullptr;
-  void *arena = nullptr;        // trace + state, one allocation
-  void *dyn_arena = nullptr;    // tables of swb_sim_set_dynamic
-  void *wt_arena = nullptr;     // tables of swb_sim_set_worker_types
+  DBuf arena;                   // trace + state, one allocation
+  DBuf dyn_arena;               // tables of swb_sim_set_dynamic
+  DBuf wt_arena;                // tables of swb_sim_set_worker_types
   int needs_dynamic = 0;        // the trace names non-static jobs: tables are required before the first round
-  unsigned char *d_chosen = nullptr;
-  size_t chosen_cap = 0;
-  unsigned char *h_pin = nullptr;   // pinned staging of the per-step outputs
-  size_t pin_cap = 0;
+  DBuf d_chosen;                // chosen / schedule of the latest step or replay
+  PinBuf h_pin;                 // pinned staging of the per-step outputs
   swb::sim::Trace T;
   swb::sim::State X;
   swb::sim::Scn *scn = nullptr;
 };
-
-#define SCK(call)                                                                                   \
-  do {                                                                                              \
-    cudaError_t e_ = (call);                                                                        \
-    if (e_ != cudaSuccess) return swb_set_error(SWB_ERR_CUDA, (std::string(#call) + ": " + cudaGetErrorString(e_)).c_str()); \
-  } while (0)
 
 static size_t al(size_t b) { return (b + 255) & ~(size_t)255; }
 
@@ -73,13 +65,8 @@ void swb_sim_destroy(swb_sim *m) {
   if (!m) return;
   cudaSetDevice(m->device);
   if (m->st) cudaStreamSynchronize(m->st);
-  if (m->arena) cudaFree(m->arena);
-  if (m->dyn_arena) cudaFree(m->dyn_arena);
-  if (m->wt_arena) cudaFree(m->wt_arena);
-  if (m->d_chosen) cudaFree(m->d_chosen);
-  if (m->h_pin) cudaFreeHost(m->h_pin);
   if (m->st) cudaStreamDestroy(m->st);
-  delete m;
+  delete m;      // the buffers free themselves
 }
 
 int swb_sim_create(int32_t device, const swb_sim_trace *tr, int32_t S, int32_t ngpus, double time_per_iteration,
@@ -131,12 +118,12 @@ int swb_sim_create(int32_t device, const swb_sim_trace *tr, int32_t S, int32_t n
                o_epoch = take(sj * 4), o_running = take(sj), o_flag = take(sj), o_fails = take(sj), o_cbs = take(sj * 4),
                o_ctotal = take(sj * 8), o_cspe = take(sj * 8), o_cthr = take(sj * 8), o_lastex = take(sj * 8),
                o_scn = take((size_t)S * sizeof(swb::sim::Scn));
-  if (e == cudaSuccess) e = cudaMalloc(&m->arena, off);
+  if (e == cudaSuccess) e = m->arena.need(off, m->st);
   if (e != cudaSuccess) {
     swb_sim_destroy(m);
     return swb_set_error(SWB_ERR_CUDA, (std::string("swb_sim_create: ") + cudaGetErrorString(e)).c_str());
   }
-  char *b = (char *)m->arena;
+  char *b = m->arena.as<char>();
   auto up = [&](size_t o, const void *src, size_t bytes) {
     return cudaMemcpyAsync(b + o, src, bytes, cudaMemcpyHostToDevice, m->st);
   };
@@ -179,43 +166,26 @@ static int sim_run(swb_sim *m, const unsigned char *d_chosen, long long stride_r
   // block size: a multiple of 32 (the reductions shuffle over full warps), one job per thread up to 256
   const int threads = m->J <= 32 ? 32 : m->J <= 64 ? 64 : m->J <= 128 ? 128 : SIM_THREADS;
   swb::sim_kernel<<<m->S, threads, 0, m->st>>>(L);
-  SCK(cudaGetLastError());
+  CK(cudaGetLastError());
   const size_t sj = (size_t)m->S * m->J;
-  const size_t need = al((size_t)m->S * sizeof(swb_sim_scn)) + al(sj) + 2 * al(sj * 4) + al(sj * 8);
-  if (need > m->pin_cap) {
-    if (m->h_pin) cudaFreeHost(m->h_pin);
-    m->h_pin = nullptr; m->pin_cap = 0;
-    SCK(cudaMallocHost((void **)&m->h_pin, need));
-    m->pin_cap = need;
-  }
-  unsigned char *p = m->h_pin;
+  CK(m->h_pin.need(al((size_t)m->S * sizeof(swb_sim_scn)) + al(sj) + 2 * al(sj * 4) + al(sj * 8)));
+  unsigned char *p = m->h_pin.as<unsigned char>();
   unsigned char *p_scn = p; p += al((size_t)m->S * sizeof(swb_sim_scn));
   unsigned char *p_st = p; p += al(sj);
   unsigned char *p_ep = p; p += al(sj * 4);
   unsigned char *p_te = p; p += al(sj * 4);
   unsigned char *p_ns = p;
-  if (scn) SCK(cudaMemcpyAsync(p_scn, m->scn, (size_t)m->S * sizeof(swb_sim_scn), cudaMemcpyDeviceToHost, m->st));
-  if (status) SCK(cudaMemcpyAsync(p_st, m->X.status, sj, cudaMemcpyDeviceToHost, m->st));
-  if (epoch) SCK(cudaMemcpyAsync(p_ep, m->X.epoch, sj * 4, cudaMemcpyDeviceToHost, m->st));
-  if (tl_end) SCK(cudaMemcpyAsync(p_te, m->X.tl_end, sj * 4, cudaMemcpyDeviceToHost, m->st));
-  if (tl_ns) SCK(cudaMemcpyAsync(p_ns, m->X.tl_ns, sj * 8, cudaMemcpyDeviceToHost, m->st));
-  SCK(cudaStreamSynchronize(m->st));
+  if (scn) CK(cudaMemcpyAsync(p_scn, m->scn, (size_t)m->S * sizeof(swb_sim_scn), cudaMemcpyDeviceToHost, m->st));
+  if (status) CK(cudaMemcpyAsync(p_st, m->X.status, sj, cudaMemcpyDeviceToHost, m->st));
+  if (epoch) CK(cudaMemcpyAsync(p_ep, m->X.epoch, sj * 4, cudaMemcpyDeviceToHost, m->st));
+  if (tl_end) CK(cudaMemcpyAsync(p_te, m->X.tl_end, sj * 4, cudaMemcpyDeviceToHost, m->st));
+  if (tl_ns) CK(cudaMemcpyAsync(p_ns, m->X.tl_ns, sj * 8, cudaMemcpyDeviceToHost, m->st));
+  CK(cudaStreamSynchronize(m->st));
   if (scn) memcpy(scn, p_scn, (size_t)m->S * sizeof(swb_sim_scn));
   if (status) memcpy(status, p_st, sj);
   if (epoch) memcpy(epoch, p_ep, sj * 4);
   if (tl_end) memcpy(tl_end, p_te, sj * 4);
   if (tl_ns) memcpy(tl_ns, p_ns, sj * 8);
-  return 0;
-}
-
-static int sim_upload(swb_sim *m, const uint8_t *chosen, size_t bytes) {
-  if (bytes > m->chosen_cap) {
-    if (m->d_chosen) cudaFree(m->d_chosen);
-    m->d_chosen = nullptr; m->chosen_cap = 0;
-    SCK(cudaMalloc((void **)&m->d_chosen, bytes));
-    m->chosen_cap = bytes;
-  }
-  SCK(cudaMemcpyAsync(m->d_chosen, chosen, bytes, cudaMemcpyHostToDevice, m->st));
   return 0;
 }
 
@@ -236,26 +206,24 @@ int swb_sim_set_dynamic(swb_sim *m, const swb_sim_dynamic *d) {
   }
   const long long np = d->pat_off[J];
   if (np > 0 && !d->pattern) return swb_set_error(SWB_ERR_ARG, "swb_sim_set_dynamic: null pattern");
-  SCK(cudaSetDevice(m->device));
+  CK(cudaSetDevice(m->device));
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off += al(bytes ? bytes : 1); return o; };
   const size_t o_mode = take((size_t)J * 4), o_max = take((size_t)J * 4), o_min = take((size_t)J * 4), o_big = take((size_t)J * 4),
                o_lock = take((size_t)J * 4), o_skip = take((size_t)J * 4), o_off = take((size_t)(J + 1) * 8),
                o_pat = take((size_t)np * 4), o_lb = take((size_t)J * K * 4), o_lt = take((size_t)J * K * 8);
-  SCK(cudaStreamSynchronize(m->st));
-  if (m->dyn_arena) cudaFree(m->dyn_arena);
-  m->dyn_arena = nullptr;
-  SCK(cudaMalloc(&m->dyn_arena, off));
-  char *b = (char *)m->dyn_arena;
+  CK(cudaStreamSynchronize(m->st));      // a launched round may still read the old tables
+  CK(m->dyn_arena.need(off, m->st));
+  char *b = m->dyn_arena.as<char>();
   auto up = [&](size_t o, const void *src, size_t bytes) {
     return bytes ? cudaMemcpyAsync(b + o, src, bytes, cudaMemcpyHostToDevice, m->st) : cudaSuccess;
   };
-  SCK(up(o_mode, d->mode, (size_t)J * 4)); SCK(up(o_max, d->bs_max, (size_t)J * 4)); SCK(up(o_min, d->bs_min, (size_t)J * 4));
-  SCK(up(o_big, d->bs_big, (size_t)J * 4)); SCK(up(o_lock, d->orig_locked, (size_t)J * 4));
-  SCK(up(o_skip, d->acc_skip, (size_t)J * 4)); SCK(up(o_off, d->pat_off, (size_t)(J + 1) * 8));
-  SCK(up(o_pat, d->pattern, (size_t)np * 4)); SCK(up(o_lb, d->lvl_bs, (size_t)J * K * 4));
-  SCK(up(o_lt, d->lvl_thr, (size_t)J * K * 8));
-  SCK(cudaStreamSynchronize(m->st));
+  CK(up(o_mode, d->mode, (size_t)J * 4)); CK(up(o_max, d->bs_max, (size_t)J * 4)); CK(up(o_min, d->bs_min, (size_t)J * 4));
+  CK(up(o_big, d->bs_big, (size_t)J * 4)); CK(up(o_lock, d->orig_locked, (size_t)J * 4));
+  CK(up(o_skip, d->acc_skip, (size_t)J * 4)); CK(up(o_off, d->pat_off, (size_t)(J + 1) * 8));
+  CK(up(o_pat, d->pattern, (size_t)np * 4)); CK(up(o_lb, d->lvl_bs, (size_t)J * K * 4));
+  CK(up(o_lt, d->lvl_thr, (size_t)J * K * 8));
+  CK(cudaStreamSynchronize(m->st));
   m->T.mode = (const int *)(b + o_mode); m->T.bs_max = (const int *)(b + o_max); m->T.bs_min = (const int *)(b + o_min);
   m->T.bs_big = (const int *)(b + o_big); m->T.orig_locked = (const int *)(b + o_lock); m->T.acc_skip = (const int *)(b + o_skip);
   m->T.pat_off = (const long long *)(b + o_off); m->T.pattern = (const int *)(b + o_pat); m->T.K = K;
@@ -275,16 +243,15 @@ int swb_sim_set_worker_types(swb_sim *m, int32_t W, const double *throughput, co
     if (ngpus[w] < 0) return swb_set_error(SWB_ERR_ARG, "swb_sim_set_worker_types: negative worker count");
   for (size_t i = 0; i < (size_t)J * W; ++i)
     if (!(throughput[i] >= 0.0)) return swb_set_error(SWB_ERR_ARG, "swb_sim_set_worker_types: throughput must be >= 0 (0 = the job cannot run on that type)");
-  SCK(cudaSetDevice(m->device));
+  CK(cudaSetDevice(m->device));
   const size_t o_thr = 0, o_cap = al((size_t)J * W * 8), total = o_cap + al((size_t)W * 4);
-  SCK(cudaStreamSynchronize(m->st));
-  if (m->wt_arena) cudaFree(m->wt_arena);
-  m->wt_arena = nullptr; m->T.thr_w = nullptr; m->T.cap_w = nullptr; m->T.W = 0;
-  SCK(cudaMalloc(&m->wt_arena, total));
-  char *b = (char *)m->wt_arena;
-  SCK(cudaMemcpyAsync(b + o_thr, throughput, (size_t)J * W * 8, cudaMemcpyHostToDevice, m->st));
-  SCK(cudaMemcpyAsync(b + o_cap, ngpus, (size_t)W * 4, cudaMemcpyHostToDevice, m->st));
-  SCK(cudaStreamSynchronize(m->st));
+  CK(cudaStreamSynchronize(m->st));      // a launched round may still read the old tables
+  m->T.thr_w = nullptr; m->T.cap_w = nullptr; m->T.W = 0;
+  CK(m->wt_arena.need(total, m->st));
+  char *b = m->wt_arena.as<char>();
+  CK(cudaMemcpyAsync(b + o_thr, throughput, (size_t)J * W * 8, cudaMemcpyHostToDevice, m->st));
+  CK(cudaMemcpyAsync(b + o_cap, ngpus, (size_t)W * 4, cudaMemcpyHostToDevice, m->st));
+  CK(cudaStreamSynchronize(m->st));
   m->T.W = W; m->T.thr_w = (const double *)(b + o_thr); m->T.cap_w = (const int *)(b + o_cap);
   return 0;
 }
@@ -293,7 +260,7 @@ int swb_sim_begin(swb_sim *m, swb_sim_scn *scn, uint8_t *status) {
   if (!m) return swb_set_error(SWB_ERR_ARG, "swb_sim_begin: null handle");
   if (m->needs_dynamic)
     return swb_set_error(SWB_ERR_STATE, "swb_sim_begin: the trace has accordion / gns jobs: call swb_sim_set_dynamic first");
-  SCK(cudaSetDevice(m->device));
+  CK(cudaSetDevice(m->device));
   m->begun = 1;
   return sim_run(m, nullptr, 0, 0, 0, 1, scn, status, nullptr, nullptr, nullptr);
 }
@@ -302,49 +269,49 @@ int swb_sim_step(swb_sim *m, const uint8_t *chosen, swb_sim_scn *scn, uint8_t *s
                  int32_t *tl_end) {
   if (!m || !chosen) return swb_set_error(SWB_ERR_ARG, "swb_sim_step: null argument");
   if (!m->begun) return swb_set_error(SWB_ERR_STATE, "swb_sim_step: call swb_sim_begin first");
-  SCK(cudaSetDevice(m->device));
+  CK(cudaSetDevice(m->device));
   const size_t sj = (size_t)m->S * m->J;
-  if (int rc = sim_upload(m, chosen, sj)) return rc;
-  return sim_run(m, m->d_chosen, 0, m->J, 1, 0, scn, status, epoch, tl_ns, tl_end);
+  CK(m->d_chosen.upload(chosen, sj, m->st));
+  return sim_run(m, m->d_chosen.as<unsigned char>(), 0, m->J, 1, 0, scn, status, epoch, tl_ns, tl_end);
 }
 
 int swb_sim_replay(swb_sim *m, const uint8_t *schedule, int32_t R, int32_t per_scenario, swb_sim_scn *scn) {
   if (!m || !schedule || R <= 0) return swb_set_error(SWB_ERR_ARG, "swb_sim_replay: null argument or R <= 0");
-  SCK(cudaSetDevice(m->device));
+  CK(cudaSetDevice(m->device));
   const size_t per_round = per_scenario ? (size_t)m->S * m->J : (size_t)m->J;
   if (per_round * (size_t)R > ((size_t)4 << 30)) return swb_set_error(SWB_ERR_ARG, "swb_sim_replay: schedule above 4 GiB");
   if (m->needs_dynamic)
     return swb_set_error(SWB_ERR_STATE, "swb_sim_replay: the trace has accordion / gns jobs: call swb_sim_set_dynamic first");
-  if (int rc = sim_upload(m, schedule, per_round * (size_t)R)) return rc;
+  CK(m->d_chosen.upload(schedule, per_round * (size_t)R, m->st));
   m->begun = 1;
-  return sim_run(m, m->d_chosen, (long long)per_round, per_scenario ? m->J : 0, R, 1, scn, nullptr, nullptr, nullptr, nullptr);
+  return sim_run(m, m->d_chosen.as<unsigned char>(), (long long)per_round, per_scenario ? m->J : 0, R, 1, scn, nullptr, nullptr, nullptr, nullptr);
 }
 
 int swb_sim_results(swb_sim *m, double *jct, int64_t *steps_run, double *run_time, double *measured_throughput) {
   if (!m) return swb_set_error(SWB_ERR_ARG, "swb_sim_results: null handle");
-  SCK(cudaSetDevice(m->device));
+  CK(cudaSetDevice(m->device));
   const size_t sj = (size_t)m->S * m->J;
-  if (jct) SCK(cudaMemcpyAsync(jct, m->X.jct, sj * 8, cudaMemcpyDeviceToHost, m->st));
-  if (steps_run) SCK(cudaMemcpyAsync(steps_run, m->X.steps_run, sj * 8, cudaMemcpyDeviceToHost, m->st));
-  if (run_time) SCK(cudaMemcpyAsync(run_time, m->X.run_time, sj * 8, cudaMemcpyDeviceToHost, m->st));
-  if (measured_throughput) SCK(cudaMemcpyAsync(measured_throughput, m->X.thr_meas, sj * 8, cudaMemcpyDeviceToHost, m->st));
-  SCK(cudaStreamSynchronize(m->st));
+  if (jct) CK(cudaMemcpyAsync(jct, m->X.jct, sj * 8, cudaMemcpyDeviceToHost, m->st));
+  if (steps_run) CK(cudaMemcpyAsync(steps_run, m->X.steps_run, sj * 8, cudaMemcpyDeviceToHost, m->st));
+  if (run_time) CK(cudaMemcpyAsync(run_time, m->X.run_time, sj * 8, cudaMemcpyDeviceToHost, m->st));
+  if (measured_throughput) CK(cudaMemcpyAsync(measured_throughput, m->X.thr_meas, sj * 8, cudaMemcpyDeviceToHost, m->st));
+  CK(cudaStreamSynchronize(m->st));
   return 0;
 }
 
 int swb_sim_job_state(swb_sim *m, int64_t *total_steps, double *throughput, int32_t *batch_size, double *exec_time,
                       double *finish_time, uint8_t *failed_attempts, uint8_t *ran) {
   if (!m) return swb_set_error(SWB_ERR_ARG, "swb_sim_job_state: null handle");
-  SCK(cudaSetDevice(m->device));
+  CK(cudaSetDevice(m->device));
   const size_t sj = (size_t)m->S * m->J;
-  if (total_steps) SCK(cudaMemcpyAsync(total_steps, m->X.ctotal, sj * 8, cudaMemcpyDeviceToHost, m->st));
-  if (throughput) SCK(cudaMemcpyAsync(throughput, m->X.cthr, sj * 8, cudaMemcpyDeviceToHost, m->st));
-  if (batch_size) SCK(cudaMemcpyAsync(batch_size, m->X.cbs, sj * 4, cudaMemcpyDeviceToHost, m->st));
-  if (exec_time) SCK(cudaMemcpyAsync(exec_time, m->X.last_ex, sj * 8, cudaMemcpyDeviceToHost, m->st));
-  if (finish_time) SCK(cudaMemcpyAsync(finish_time, m->X.fin, sj * 8, cudaMemcpyDeviceToHost, m->st));
-  if (failed_attempts) SCK(cudaMemcpyAsync(failed_attempts, m->X.fails, sj, cudaMemcpyDeviceToHost, m->st));
-  if (ran) SCK(cudaMemcpyAsync(ran, m->X.ranprev, sj, cudaMemcpyDeviceToHost, m->st));
-  SCK(cudaStreamSynchronize(m->st));
+  if (total_steps) CK(cudaMemcpyAsync(total_steps, m->X.ctotal, sj * 8, cudaMemcpyDeviceToHost, m->st));
+  if (throughput) CK(cudaMemcpyAsync(throughput, m->X.cthr, sj * 8, cudaMemcpyDeviceToHost, m->st));
+  if (batch_size) CK(cudaMemcpyAsync(batch_size, m->X.cbs, sj * 4, cudaMemcpyDeviceToHost, m->st));
+  if (exec_time) CK(cudaMemcpyAsync(exec_time, m->X.last_ex, sj * 8, cudaMemcpyDeviceToHost, m->st));
+  if (finish_time) CK(cudaMemcpyAsync(finish_time, m->X.fin, sj * 8, cudaMemcpyDeviceToHost, m->st));
+  if (failed_attempts) CK(cudaMemcpyAsync(failed_attempts, m->X.fails, sj, cudaMemcpyDeviceToHost, m->st));
+  if (ran) CK(cudaMemcpyAsync(ran, m->X.ranprev, sj, cudaMemcpyDeviceToHost, m->st));
+  CK(cudaStreamSynchronize(m->st));
   return 0;
 }
 

@@ -19,7 +19,6 @@
 // shuffles + one barrier.  The dense J x T placement of the counts is place.cu.
 #include <cooperative_groups.h>
 #include <math.h>
-#include <stdlib.h>
 
 #include "swb_common.cuh"
 #include "swb_internal.h"
@@ -711,8 +710,7 @@ __global__ void __launch_bounds__(NT, 1) solve_kernel(SolveLaunch L) {
   if constexpr (CL > 1) cg::this_cluster().sync();   // nobody leaves while its exchange slots may still be read
 }
 
-static int g_solve_nt = 1024;   // threads per CTA of the shared-memory variant (SWB_SOLVE_NT=512 for experiments)
-static int g_solve_cl = 8;      // CTAs per scenario on the latency path (SWB_SOLVE_CLUSTER=1 switches the cluster off)
+static int g_solve_cl = 8;      // CTAs per scenario on the latency path (SWB_OPT_SOLVE_CLUSTER = 1 switches the cluster off)
 
 void set_solve_cluster(int v) { g_solve_cl = (v == 8) ? 8 : 1; }
 
@@ -733,12 +731,7 @@ cudaError_t launch_solve(const SolveLaunch &L, cudaStream_t st, int nbases) {
     cudaError_t e = cudaFuncGetAttributes(&fa, solve_kernel<true, 1024, 1>);
     if (e != cudaSuccess) return e;
     if ((e = set_smem_attr(solve_kernel<true, 1024, 1>, (int)fa.sharedSizeBytes)) != cudaSuccess) return e;
-    if ((e = set_smem_attr(solve_kernel<true, 512, 1>, (int)fa.sharedSizeBytes)) != cudaSuccess) return e;
     if ((e = set_smem_attr(solve_kernel<true, 512, 8>, (int)fa.sharedSizeBytes)) != cudaSuccess) return e;
-    const char *env = getenv("SWB_SOLVE_NT");
-    if (env) g_solve_nt = atoi(env) == 512 ? 512 : 1024;
-    env = getenv("SWB_SOLVE_CLUSTER");
-    if (env) g_solve_cl = atoi(env) == 8 ? 8 : 1;
     attr_set = true;
   }
   // Latency path: few scenarios of many jobs leave most of the 148 SMs idle with one CTA per scenario — a cluster of
@@ -760,10 +753,9 @@ cudaError_t launch_solve(const SolveLaunch &L, cudaStream_t st, int nbases) {
   size_t smem = smem_fixed;
   if (L.jobs_in_smem) smem += (size_t)L.J * (2 * sizeof(double) + 5 * (size_t)nbases + 3);
   int nt = ((L.J + 31) / 32) * 32;
-  if (nt > g_solve_nt) nt = g_solve_nt;
+  if (nt > 1024) nt = 1024;
   if (nt < 64) nt = 64;
   if (!L.jobs_in_smem) solve_kernel<false, 1024, 1><<<L.S, nt, smem, st>>>(L);
-  else if (g_solve_nt == 512) solve_kernel<true, 512, 1><<<L.S, nt, smem, st>>>(L);
   else solve_kernel<true, 1024, 1><<<L.S, nt, smem, st>>>(L);
   return cudaGetLastError();
 }

@@ -3,6 +3,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <string>
+
 #include "../../include/swb200.h"
 
 #define SWB_SOLVE_THREADS 1024
@@ -14,8 +16,81 @@
 #define SWB_MAX_REPLAN 6             /* packing-feedback re-solves (caps written by place_kernel) */
 #define SWB_MAX_J 8192              /* 13 index bits in the placement sort key */
 
-// error hook for the .cu files that carry their own extern "C" entry points (sim.cu): sets swb_last_error()
+// sets swb_last_error() and returns `code`
 extern "C" int swb_set_error(int code, const char *msg);
+
+// return SWB_ERR_CUDA from the enclosing entry point when a CUDA call fails
+#define CK(call)                                                                                   \
+  do {                                                                                             \
+    cudaError_t e_ = (call);                                                                       \
+    if (e_ != cudaSuccess)                                                                         \
+      return swb_set_error(SWB_ERR_CUDA, (std::string(#call) + ": " + cudaGetErrorString(e_)).c_str()); \
+  } while (0)
+
+// capacity after growing `cap` to hold `bytes`: doubling from 256 bytes
+inline size_t swb_grow_cap(size_t cap, size_t bytes) {
+  size_t ncap = cap ? cap : 256;
+  while (ncap < bytes) ncap *= 2;
+  return ncap;
+}
+
+// Grow-only device buffer, freed by its destructor.  need() with `keep` preserves the old contents and zeroes the
+// new tail (the resident job table grows in place that way); without it the contents are undefined after growth.
+struct DBuf {
+  void *p = nullptr;
+  size_t cap = 0;
+  DBuf() = default;
+  DBuf(const DBuf &) = delete;
+  DBuf &operator=(const DBuf &) = delete;
+  ~DBuf() { if (p) cudaFree(p); }
+  cudaError_t need(size_t bytes, cudaStream_t st, bool keep = false) {
+    if (bytes <= cap) return cudaSuccess;
+    const size_t ncap = swb_grow_cap(cap, bytes);
+    void *np = nullptr;
+    cudaError_t e = cudaMalloc(&np, ncap);
+    if (e != cudaSuccess) return e;
+    if (keep && p && cap) {
+      e = cudaMemcpyAsync(np, p, cap, cudaMemcpyDeviceToDevice, st);
+      if (e != cudaSuccess) return e;
+      e = cudaStreamSynchronize(st);
+      if (e != cudaSuccess) return e;
+    }
+    if (keep && ncap > cap) {
+      e = cudaMemsetAsync((char *)np + cap, 0, ncap - cap, st);
+      if (e != cudaSuccess) return e;
+    }
+    if (p) cudaFree(p);
+    p = np; cap = ncap;
+    return cudaSuccess;
+  }
+  // grow to `bytes`, then copy `bytes` from the host on `st`
+  cudaError_t upload(const void *src, size_t bytes, cudaStream_t st) {
+    const cudaError_t e = need(bytes, st);
+    return e != cudaSuccess ? e : cudaMemcpyAsync(p, src, bytes, cudaMemcpyHostToDevice, st);
+  }
+  template <class T> T *as() { return reinterpret_cast<T *>(p); }
+};
+
+// Grow-only pinned host buffer (staging of truly asynchronous copies), freed by its destructor; the contents are
+// undefined after growth.
+struct PinBuf {
+  void *p = nullptr;
+  size_t cap = 0;
+  PinBuf() = default;
+  PinBuf(const PinBuf &) = delete;
+  PinBuf &operator=(const PinBuf &) = delete;
+  ~PinBuf() { if (p) cudaFreeHost(p); }
+  cudaError_t need(size_t bytes) {
+    if (bytes <= cap) return cudaSuccess;
+    const size_t ncap = swb_grow_cap(cap, bytes);
+    if (p) cudaFreeHost(p);
+    p = nullptr; cap = 0;
+    const cudaError_t e = cudaMallocHost(&p, ncap);
+    if (e == cudaSuccess) cap = ncap;
+    return e;
+  }
+  template <class T> T *as() { return reinterpret_cast<T *>(p); }
+};
 
 namespace swb {
 

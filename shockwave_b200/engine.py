@@ -41,6 +41,7 @@ class Result(C.Structure):
 
 
 class SolveArgs(C.Structure):
+    """swb_solve_args (include/swb200.h)."""
     _fields_ = [("S", C.c_int32), ("J", C.c_int32), ("per_scenario_jobs", C.c_int32),
                 ("on_device", C.c_int32), ("prm", C.POINTER(Params)),
                 ("g", C.c_void_p), ("E", C.c_void_p), ("c", C.c_void_p),
@@ -50,6 +51,7 @@ class SolveArgs(C.Structure):
 
 
 class RoundArgs(C.Structure):
+    """swb_round_args (include/swb200.h)."""
     _fields_ = [("J", C.c_int32), ("reestimate_share", C.c_int32), ("gavel_round_duration", C.c_double),
                 ("slots", C.c_void_p), ("epoch_progress", C.c_void_p), ("meas_nsamples", C.c_void_p),
                 ("meas_end_round", C.c_void_p), ("x", C.c_void_p), ("backfill", C.c_void_p),
@@ -57,10 +59,91 @@ class RoundArgs(C.Structure):
                 ("xmask", C.c_void_p), ("bfmask", C.c_void_p)]
 
 
-EXPORTS = ["swb_create", "swb_destroy", "swb_last_error", "swb_version", "swb_stream", "swb_sync",
-           "swb_solve", "swb_job_add", "swb_job_remove", "swb_job_table_stats", "swb_job_set_gbm", "swb_gbm_ensemble", "swb_gavel_round", "swb_round_solve", "swb_forecast",
-           "swb_forecast_commit", "swb_last_timings", "swb_policy_pooled", "swb_policy_hetero", "swb_policy_waterfill_step", "swb_gbm_forecast", "swb_market_pgd", "swb_set_option", "swb_allox_assign", "swb_lp_solve",
-           "swb_sim_create", "swb_sim_destroy", "swb_sim_begin", "swb_sim_step", "swb_sim_replay", "swb_sim_results", "swb_sim_set_dynamic", "swb_sim_job_state", "swb_sim_set_worker_types"]
+class MarketArgs(C.Structure):
+    """swb_market_args (include/swb200.h)."""
+    _fields_ = [("S", C.c_int32), ("J", C.c_int32), ("W", C.c_int32), ("T", C.c_int32),
+                ("per_scenario_jobs", C.c_int32), ("on_device", C.c_int32), ("iters", C.c_int32),
+                ("coarse_iters", C.c_int32), ("warm_start", C.c_int32), ("primal_weight", C.c_float), ("utility", C.c_int32),
+                ("prm", C.POINTER(Params)), ("g", C.c_void_p), ("E", C.c_void_p), ("c", C.c_void_p),
+                ("dbar", C.c_void_p), ("rem", C.c_void_p), ("rate", C.c_void_p), ("Gw", C.c_void_p),
+                ("cap", C.c_void_p), ("X", C.c_void_p), ("obj", C.c_void_p), ("dense_ms", C.POINTER(C.c_float))]
+
+
+class GavelRoundArgs(C.Structure):
+    """swb_gavel_round_args (include/swb200.h)."""
+    _fields_ = [("J", C.c_int32), ("W", C.c_int32), ("flags", C.c_int32)] + \
+               [(n, C.c_void_p) for n in ("type_order", "capacity", "alloc", "job_time", "thr", "deficit",
+                                          "worker_time", "sf", "nworkers", "worker_ids", "prev_type", "prev_off",
+                                          "prev_local", "prio", "n_sel", "sel_jobs")] + \
+               [("n_assigned", C.POINTER(C.c_int32))] + \
+               [(n, C.c_void_p) for n in ("assign_job", "assign_off", "assign_workers")]
+
+
+class SimTrace(C.Structure):
+    """swb_sim_trace (include/swb200.h)."""
+    _fields_ = [("J", C.c_int32), ("reserved", C.c_int32), ("arrival", C.c_void_p), ("total_steps", C.c_void_p),
+                ("scale_factor", C.c_void_p), ("throughput", C.c_void_p), ("duration", C.c_void_p),
+                ("batch_size", C.c_void_p), ("dataset_len", C.c_void_p), ("adaptation_mode", C.c_void_p)]
+
+
+class SimDynamic(C.Structure):
+    """swb_sim_dynamic (include/swb200.h)."""
+    _fields_ = [("mode", C.c_void_p), ("bs_max", C.c_void_p), ("bs_min", C.c_void_p), ("bs_big", C.c_void_p),
+                ("orig_locked", C.c_void_p), ("acc_skip", C.c_void_p), ("pat_off", C.c_void_p), ("pattern", C.c_void_p),
+                ("n_levels", C.c_int32), ("reserved", C.c_int32), ("lvl_bs", C.c_void_p), ("lvl_thr", C.c_void_p)]
+
+
+class SimScn(C.Structure):
+    """swb_sim_scn (include/swb200.h)."""
+    _fields_ = [("now", C.c_double), ("round_start", C.c_double), ("round_end", C.c_double), ("rounds", C.c_int32),
+                ("remaining", C.c_int32), ("n_active", C.c_int32), ("done", C.c_int32), ("err", C.c_int32),
+                ("reserved", C.c_int32)]
+
+
+SCN_DTYPE = np.dtype([("now", "f8"), ("round_start", "f8"), ("round_end", "f8"), ("rounds", "i4"), ("remaining", "i4"),
+                      ("n_active", "i4"), ("done", "i4"), ("err", "i4"), ("reserved", "i4")])   # numpy view of SimScn
+assert SCN_DTYPE.itemsize == C.sizeof(SimScn) == 48
+
+# Every function include/swb200.h declares: name -> (restype, argtypes).  load_library() binds the whole table;
+# tests/test_abi_and_host.py checks it against the header's prototypes.
+_P, _I32, _I64, _F64, _PF64 = C.c_void_p, C.c_int32, C.c_int64, C.c_double, C.POINTER(C.c_double)
+ABI = {
+    "swb_create": (C.c_int, [C.POINTER(C.c_void_p), C.c_int]),
+    "swb_destroy": (None, [_P]),
+    "swb_last_error": (C.c_char_p, []),
+    "swb_version": (C.c_int, []),
+    "swb_stream": (C.c_void_p, [_P]),
+    "swb_sync": (C.c_int, [_P]),
+    "swb_set_option": (C.c_int, [_P, _I32, _I32]),
+    "swb_solve": (C.c_int, [_P, C.POINTER(SolveArgs)]),
+    "swb_job_add": (C.c_int, [_P, _I32, _I32, _I32, _F64, _F64, _P, _P]),
+    "swb_job_remove": (C.c_int, [_P, _I32]),
+    "swb_job_table_stats": (C.c_int, [_P, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "swb_job_set_gbm": (C.c_int, [_P, _I32, _F64, _F64]),
+    "swb_round_solve": (C.c_int, [_P, C.POINTER(Params), C.POINTER(RoundArgs)]),
+    "swb_forecast": (C.c_int, [_P, C.POINTER(Params), C.POINTER(RoundArgs)] + [_P] * 5),
+    "swb_forecast_commit": (C.c_int, [_P, _I32, _I32, _P]),
+    "swb_policy_pooled": (C.c_int, [_P, _I32, _I32, _F64] + [_P] * 6 + [_PF64]),
+    "swb_policy_hetero": (C.c_int, [_P, _I32, _I32, _I32] + [_P] * 7 + [_PF64, _P]),
+    "swb_policy_waterfill_step": (C.c_int, [_P, _I32, _I32] + [_P] * 6 + [_F64, _F64, _P, _PF64, _P, _P]),
+    "swb_lp_solve": (C.c_int, [_P] + [_I32] * 4 + [_P] * 5 + [_I32] + [_P] * 4),
+    "swb_allox_assign": (C.c_int, [_P, _I32, _I32, _I32] + [_P] * 4 + [_PF64]),
+    "swb_gavel_round": (C.c_int, [_P, C.POINTER(GavelRoundArgs)]),
+    "swb_gbm_forecast": (C.c_int, [_P, _I32] + [_P] * 4 + [_I64, _I64, C.c_uint64, _P, _I32]),
+    "swb_gbm_ensemble": (C.c_int, [_P, _I32, _I32, _F64, _P, _P, _P]),
+    "swb_market_pgd": (C.c_int, [_P, C.POINTER(MarketArgs)]),
+    "swb_sim_set_dynamic": (C.c_int, [_P, C.POINTER(SimDynamic)]),
+    "swb_sim_set_worker_types": (C.c_int, [_P, _I32, _P, _P]),
+    "swb_sim_create": (C.c_int, [_I32, C.POINTER(SimTrace), _I32, _I32, _F64, _F64, C.POINTER(C.c_void_p)]),
+    "swb_sim_destroy": (None, [_P]),
+    "swb_sim_begin": (C.c_int, [_P, _P, _P]),
+    "swb_sim_step": (C.c_int, [_P] * 7),
+    "swb_sim_replay": (C.c_int, [_P, _P, _I32, _I32, _P]),
+    "swb_sim_results": (C.c_int, [_P] * 5),
+    "swb_sim_job_state": (C.c_int, [_P] * 8),
+    "swb_last_timings": (C.c_int, [_P, _PF64, _PF64, C.POINTER(C.c_int32)]),
+}
+EXPORTS = list(ABI)
 
 _lib = None
 
@@ -75,33 +158,9 @@ def load_library():
             f"{LIB_PATH} is missing: build it with `python -c 'import __graft_entry__ as g; g.build()'` "
             "(there is no CPU fallback for the shockwave_b200 solver)")
     lib = C.CDLL(LIB_PATH)
-    lib.swb_create.argtypes = [C.POINTER(C.c_void_p), C.c_int]
-    lib.swb_create.restype = C.c_int
-    lib.swb_destroy.argtypes = [C.c_void_p]
-    lib.swb_destroy.restype = None
-    lib.swb_last_error.restype = C.c_char_p
-    lib.swb_version.restype = C.c_int
-    lib.swb_stream.argtypes = [C.c_void_p]
-    lib.swb_stream.restype = C.c_void_p
-    lib.swb_sync.argtypes = [C.c_void_p]
-    lib.swb_sync.restype = C.c_int
-    lib.swb_solve.argtypes = [C.c_void_p, C.POINTER(SolveArgs)]
-    lib.swb_solve.restype = C.c_int
-    lib.swb_job_add.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_double,
-                                C.c_void_p, C.c_void_p]
-    lib.swb_job_add.restype = C.c_int
-    lib.swb_job_remove.argtypes = [C.c_void_p, C.c_int32]
-    lib.swb_job_remove.restype = C.c_int
-    lib.swb_round_solve.argtypes = [C.c_void_p, C.POINTER(Params), C.POINTER(RoundArgs)]
-    lib.swb_round_solve.restype = C.c_int
-    lib.swb_forecast.argtypes = [C.c_void_p, C.POINTER(Params), C.POINTER(RoundArgs)] + [C.c_void_p] * 5
-    lib.swb_forecast.restype = C.c_int
-    lib.swb_forecast_commit.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]
-    lib.swb_forecast_commit.restype = C.c_int
-    lib.swb_last_timings.argtypes = [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_int32)]
-    lib.swb_last_timings.restype = C.c_int
-    lib.swb_gbm_forecast.argtypes = [C.c_void_p, C.c_int32] + [C.c_void_p] * 4 + [C.c_int64, C.c_int64, C.c_uint64, C.c_void_p, C.c_int32]
-    lib.swb_gbm_forecast.restype = C.c_int
+    for name, (restype, argtypes) in ABI.items():
+        fn = getattr(lib, name)
+        fn.restype, fn.argtypes = restype, argtypes
     _lib = lib
     return lib
 
@@ -220,14 +279,11 @@ class Engine:
         self._check(self.lib.swb_job_remove(self.h, int(slot)), "swb_job_remove")
 
     def job_set_gbm(self, slot, mu, sigma):
-        self.lib.swb_job_set_gbm.argtypes = [C.c_void_p, C.c_int32, C.c_double, C.c_double]
         self._check(self.lib.swb_job_set_gbm(self.h, int(slot), float(mu), float(sigma)), "swb_job_set_gbm")
 
     def gbm_ensemble(self, S, J, P_total, sums_device_ptr, z, rem_out_device_ptr):
         z = np.ascontiguousarray(z, dtype=np.float64)
         assert len(z) == S
-        self.lib.swb_gbm_ensemble.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_double, C.c_void_p, C.c_void_p,
-                                              C.c_void_p]
         self._check(self.lib.swb_gbm_ensemble(self.h, int(S), int(J), float(P_total), C.c_void_p(int(sums_device_ptr)),
                                               _ptr(z), C.c_void_p(int(rem_out_device_ptr))), "swb_gbm_ensemble")
 
@@ -261,20 +317,10 @@ class Engine:
         n_sel = np.zeros(W, dtype=np.int32); sel_jobs = np.zeros((W, J), dtype=np.int32)
         n_asg = C.c_int32(); a_job = np.zeros(J, dtype=np.int32); a_off = np.zeros(J + 1, dtype=np.int32)
         a_w = np.zeros(max(1, int(nworkers.sum())), dtype=np.int32)
-
-        class Args(C.Structure):
-            _fields_ = [("J", C.c_int32), ("W", C.c_int32), ("flags", C.c_int32)] + \
-                       [(n, C.c_void_p) for n in ("type_order", "capacity", "alloc", "job_time", "thr", "deficit",
-                                                  "worker_time", "sf", "nworkers", "worker_ids", "prev_type", "prev_off",
-                                                  "prev_local", "prio", "n_sel", "sel_jobs")] + \
-                       [("n_assigned", C.POINTER(C.c_int32))] + \
-                       [(n, C.c_void_p) for n in ("assign_job", "assign_off", "assign_workers")]
-        a = Args(J, W, (1 if isolated_plus else 0) | (2 if fifo else 0), _ptr(type_order), _ptr(capacity), _ptr(alloc),
+        a = GavelRoundArgs(J, W, (1 if isolated_plus else 0) | (2 if fifo else 0), _ptr(type_order), _ptr(capacity), _ptr(alloc),
                  _ptr(job_time), _ptr(thr), _ptr(deficit), _ptr(worker_time), _ptr(sf), _ptr(nworkers), _ptr(wids),
                  _ptr(prev_type), _ptr(prev_off), _ptr(prev_local), _ptr(prio), _ptr(n_sel), _ptr(sel_jobs),
                  C.pointer(n_asg), _ptr(a_job), _ptr(a_off), _ptr(a_w))
-        self.lib.swb_gavel_round.argtypes = [C.c_void_p, C.c_void_p]
-        self.lib.swb_gavel_round.restype = C.c_int
         self._check(self.lib.swb_gavel_round(self.h, C.byref(a)), "swb_gavel_round")
         sel = {int(type_order[ti]): sel_jobs[ti, :n_sel[ti]].tolist() for ti in range(W)}
         asg = [(int(a_job[s]), tuple(a_w[a_off[s]:a_off[s + 1]].tolist())) for s in range(n_asg.value)]
@@ -282,7 +328,6 @@ class Engine:
 
     def job_table_stats(self):
         used, holes = C.c_int64(), C.c_int64()
-        self.lib.swb_job_table_stats.argtypes = [C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
         self._check(self.lib.swb_job_table_stats(self.h, C.byref(used), C.byref(holes)), "swb_job_table_stats")
         return dict(used_rows=used.value, hole_rows=holes.value)
 
@@ -336,7 +381,6 @@ class Engine:
         self._check(self.lib.swb_sync(self.h), "swb_sync")
 
     def set_option(self, option, value):
-        self.lib.swb_set_option.argtypes = [C.c_void_p, C.c_int32, C.c_int32]
         self._check(self.lib.swb_set_option(self.h, int(option), int(value)), "swb_set_option")
 
     def allox_assign(self, p, t, wtype):
@@ -347,9 +391,6 @@ class Engine:
         n = len(wtype)
         cols = np.zeros(m, dtype=np.int32)
         tot = C.c_double()
-        self.lib.swb_allox_assign.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32] + [C.c_void_p] * 4 + \
-                                             [C.POINTER(C.c_double)]
-        self.lib.swb_allox_assign.restype = C.c_int
         self._check(self.lib.swb_allox_assign(self.h, m, n, W, _ptr(p), _ptr(t), _ptr(wtype), _ptr(cols),
                                               C.byref(tot)), "swb_allox_assign")
         return cols, tot.value
@@ -371,9 +412,6 @@ class Engine:
         stats = np.zeros((S, 4), dtype=np.int32)
         if max_iter <= 0:
             max_iter = 50 * (m + n) + 1000
-        self.lib.swb_lp_solve.argtypes = [C.c_void_p] + [C.c_int32] * 4 + [C.c_void_p] * 5 + [C.c_int32] + \
-                                         [C.c_void_p] * 4
-        self.lib.swb_lp_solve.restype = C.c_int
         self._check(self.lib.swb_lp_solve(self.h, S, m, n, nnz, _ptr(colp), _ptr(rowi), _ptr(val), _ptr(c), _ptr(b),
                                           int(max_iter), _ptr(x), _ptr(obj), _ptr(status), _ptr(stats)),
                     "swb_lp_solve")
@@ -410,16 +448,6 @@ class Engine:
         return out
 
 
-class MarketArgs(C.Structure):
-    """swb_market_args (include/swb200.h)."""
-    _fields_ = [("S", C.c_int32), ("J", C.c_int32), ("W", C.c_int32), ("T", C.c_int32),
-                ("per_scenario_jobs", C.c_int32), ("on_device", C.c_int32), ("iters", C.c_int32),
-                ("coarse_iters", C.c_int32), ("warm_start", C.c_int32), ("primal_weight", C.c_float), ("utility", C.c_int32),
-                ("prm", C.POINTER(Params)), ("g", C.c_void_p), ("E", C.c_void_p), ("c", C.c_void_p),
-                ("dbar", C.c_void_p), ("rem", C.c_void_p), ("rate", C.c_void_p), ("Gw", C.c_void_p),
-                ("cap", C.c_void_p), ("X", C.c_void_p), ("obj", C.c_void_p), ("dense_ms", C.POINTER(C.c_float))]
-
-
 def market_pgd(eng, params, g, E, c, dbar, rem, rate, Gw, X, iters, coarse_iters=0, primal_weight=0.0, cap=None,
                warm_start=False, device_ptrs=None, utility=0):
     """Dense primal-dual price-response iterations on X[S,J,W,T] (fp32): `coarse_iters` on the time-coarsened tensor,
@@ -428,10 +456,6 @@ def market_pgd(eng, params, g, E, c, dbar, rem, rate, Gw, X, iters, coarse_iters
     resident data.  Gw [W] workers per type, or cap [W,T] workers per type and round.
     Returns (obj[S,3] = objective, makespan, capacity violation before the final repair ; ms of the last dense pass)."""
     lib = eng.lib
-    if not getattr(lib, "_mk_bound", False):
-        lib.swb_market_pgd.argtypes = [C.c_void_p, C.POINTER(MarketArgs)]
-        lib.swb_market_pgd.restype = C.c_int
-        lib._mk_bound = True
     plist = params if isinstance(params, (list, tuple)) else [params]
     S = len(plist)
     a = MarketArgs()

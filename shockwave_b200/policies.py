@@ -50,11 +50,6 @@ def _engine():
 def _pooled(mode, N, coef, sf, t=None, n=None, den=None):
     eng = _engine()
     lib = eng.lib
-    if not getattr(lib, "_pol_bound", False):
-        lib.swb_policy_pooled.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_double] + [C.c_void_p] * 6 + \
-                                         [C.POINTER(C.c_double)]
-        lib.swb_policy_pooled.restype = C.c_int
-        lib._pol_bound = True
     arr = lambda a: None if a is None else np.ascontiguousarray(a, dtype=np.float64)
     coef, sf, t, n, den = arr(coef), arr(sf), arr(t), arr(n), arr(den)
     J = len(coef)
@@ -78,11 +73,6 @@ def _hetero(mode, N, a, sf, t=None, n=None, den=None):
         return out
     eng = _engine()
     lib = eng.lib
-    if not getattr(lib, "_het_bound", False):
-        lib.swb_policy_hetero.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32] + [C.c_void_p] * 7 + \
-                                         [C.POINTER(C.c_double), C.c_void_p]
-        lib.swb_policy_hetero.restype = C.c_int
-        lib._het_bound = True
     arr = lambda v: None if v is None else np.ascontiguousarray(v, dtype=np.float64)
     a, sf, t, n, den, N = arr(a), arr(sf), arr(t), arr(n), arr(den), arr(N)
     J, W = a.shape
@@ -253,12 +243,6 @@ def _waterfill_step(N, thr, sf, prop, lower, mult, M, slack=1.0001):
     Returns (x[J,W], c, z[J]) or (None, None, None) when the LP has no feasible point."""
     eng = _engine()
     lib = eng.lib
-    if not getattr(lib, "_wf_bound", False):
-        lib.swb_policy_waterfill_step.argtypes = [C.c_void_p, C.c_int32, C.c_int32] + [C.c_void_p] * 6 + \
-                                                 [C.c_double, C.c_double, C.c_void_p, C.POINTER(C.c_double),
-                                                  C.c_void_p, C.c_void_p]
-        lib.swb_policy_waterfill_step.restype = C.c_int
-        lib._wf_bound = True
     arr = lambda v: np.ascontiguousarray(v, dtype=np.float64)
     N, thr, sf, prop, lower, mult = arr(N), arr(thr), arr(sf), arr(prop), arr(lower), arr(mult)
     J, W = thr.shape

@@ -21,21 +21,10 @@ from collections import OrderedDict
 import numpy as np
 
 from . import engine as _eng
+from .engine import SCN_DTYPE, SimDynamic, SimTrace
 from .scheduler import ShockwaveScheduler
 
 REOPT_ROUNDS = 8          # scheduler/scheduler.py:71
-
-
-class SimTrace(C.Structure):
-    _fields_ = [("J", C.c_int32), ("reserved", C.c_int32), ("arrival", C.c_void_p), ("total_steps", C.c_void_p),
-                ("scale_factor", C.c_void_p), ("throughput", C.c_void_p), ("duration", C.c_void_p),
-                ("batch_size", C.c_void_p), ("dataset_len", C.c_void_p), ("adaptation_mode", C.c_void_p)]
-
-
-class SimDynamic(C.Structure):
-    _fields_ = [("mode", C.c_void_p), ("bs_max", C.c_void_p), ("bs_min", C.c_void_p), ("bs_big", C.c_void_p),
-                ("orig_locked", C.c_void_p), ("acc_skip", C.c_void_p), ("pat_off", C.c_void_p), ("pattern", C.c_void_p),
-                ("n_levels", C.c_int32), ("reserved", C.c_int32), ("lvl_bs", C.c_void_p), ("lvl_thr", C.c_void_p)]
 
 
 def pack_dynamic_tables(dyn, J):
@@ -58,42 +47,6 @@ def pack_dynamic_tables(dyn, J):
     return a
 
 
-class SimScn(C.Structure):
-    _fields_ = [("now", C.c_double), ("round_start", C.c_double), ("round_end", C.c_double), ("rounds", C.c_int32),
-                ("remaining", C.c_int32), ("n_active", C.c_int32), ("done", C.c_int32), ("err", C.c_int32),
-                ("reserved", C.c_int32)]
-
-
-SCN_DTYPE = np.dtype([("now", "f8"), ("round_start", "f8"), ("round_end", "f8"), ("rounds", "i4"), ("remaining", "i4"),
-                      ("n_active", "i4"), ("done", "i4"), ("err", "i4"), ("reserved", "i4")])
-assert SCN_DTYPE.itemsize == C.sizeof(SimScn) == 48
-
-_bound = False
-
-
-def _lib():
-    global _bound
-    lib = _eng.load_library()
-    if not _bound:
-        lib.swb_sim_create.argtypes = [C.c_int32, C.POINTER(SimTrace), C.c_int32, C.c_int32, C.c_double, C.c_double,
-                                       C.POINTER(C.c_void_p)]
-        lib.swb_sim_destroy.argtypes = [C.c_void_p]
-        lib.swb_sim_destroy.restype = None
-        lib.swb_sim_begin.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
-        lib.swb_sim_step.argtypes = [C.c_void_p] * 7
-        lib.swb_sim_replay.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]
-        lib.swb_sim_results.argtypes = [C.c_void_p] * 5
-        lib.swb_sim_set_dynamic.argtypes = [C.c_void_p, C.POINTER(SimDynamic)]
-        lib.swb_sim_job_state.argtypes = [C.c_void_p] * 8
-        lib.swb_sim_job_state.restype = C.c_int
-        lib.swb_sim_set_worker_types.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]
-        lib.swb_sim_set_worker_types.restype = C.c_int
-        for f in ("swb_sim_set_dynamic", "swb_sim_create", "swb_sim_begin", "swb_sim_step", "swb_sim_replay", "swb_sim_results"):
-            getattr(lib, f).restype = C.c_int
-        _bound = True
-    return lib
-
-
 TRACE_KEYS = (("arrival", np.float64), ("total_steps", np.int64), ("scale_factor", np.int32), ("throughput", np.float64),
               ("duration", np.float64), ("batch_size", np.int32), ("dataset_len", np.int64))
 
@@ -103,7 +56,7 @@ class DeviceSim:
     `adaptation_mode` ([J] int, 0 = static)."""
 
     def __init__(self, trace, S, ngpus, time_per_iteration=120.0, round_duration=None, device=0):
-        self._lib = _lib()
+        self._lib = _eng.load_library()
         self._h = None
         self.S, self.J = int(S), len(trace["arrival"])
         self._arr = {k: np.ascontiguousarray(trace[k], dtype=dt) for k, dt in TRACE_KEYS}

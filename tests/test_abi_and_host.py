@@ -3,6 +3,8 @@ without a GPU), struct layouts agree, and the host state machine of the drop-in 
 import ctypes as C
 import os
 import re
+import shutil
+import subprocess
 from collections import OrderedDict
 
 import numpy as np
@@ -14,10 +16,47 @@ from shockwave_b200.scheduler import ShockwaveScheduler, schedules_from_matrices
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def _header_functions():
+def _header_text():
     txt = open(os.path.join(ROOT, "include", "swb200.h")).read()
     txt = re.sub(r"/\*.*?\*/", "", txt, flags=re.S)
-    return sorted(set(re.findall(r"\b(swb_[a-z_0-9]+)\s*\(", txt)))
+    return re.sub(r"^\s*#.*$", "", txt, flags=re.M)
+
+
+def _header_functions():
+    return sorted(set(re.findall(r"\b(swb_[a-z_0-9]+)\s*\(", _header_text())))
+
+
+def _header_prototypes():
+    """{name: (return type, [parameter types])} of every function the header declares."""
+    protos = {}
+    for ret, name, params in re.findall(r"(?:^|(?<=[;{}]))\s*([^;{}()]*?)\b(swb_[a-z_0-9]+)\s*\(([^()]*)\)\s*;",
+                                        _header_text()):
+        params = [p.strip() for p in params.split(",")]
+        if params == ["void"]:
+            params = []
+        # drop the parameter name: what is left is its type
+        protos[name] = (ret.strip(), [re.sub(r"\b[A-Za-z_]\w*$", "", p).strip() or p for p in params])
+    return protos
+
+
+def _c_kind(ctype):
+    if "*" in ctype:
+        return "ptr"
+    base = ctype.replace("const", "").strip()
+    return {"void": "void", "int": "i32", "int32_t": "i32", "int64_t": "i64", "uint64_t": "u64",
+            "double": "f64", "float": "f32"}[base]
+
+
+def _ctypes_kind(t):
+    if t is None:
+        return "void"
+    if issubclass(t, C._Pointer):
+        return "ptr"
+    code = {"P": "ptr", "z": "ptr", "d": "f64", "f": "f32"}.get(t._type_)
+    if code:
+        return code
+    signed = t._type_.islower()
+    return {4: "i32" if signed else "u32", 8: "i64" if signed else "u64"}[C.sizeof(t)]
 
 
 def test_library_exports_every_declared_symbol():
@@ -29,11 +68,44 @@ def test_library_exports_every_declared_symbol():
     assert sorted(engine.EXPORTS) == names
 
 
-def test_struct_layouts_match_header():
-    # sizes implied by include/swb200.h (4 int32, 4 double, 2 x 16 double ; 6 int32 + 5 double)
-    assert C.sizeof(engine.Params) == 16 + 32 + 2 * 16 * 8
-    assert C.sizeof(engine.Result) == 24 + 5 * 8
+def test_function_signatures_match_header():
+    protos = _header_prototypes()
+    assert sorted(protos) == _header_functions()
+    for name, (ret, params) in protos.items():
+        restype, argtypes = engine.ABI[name]
+        assert _ctypes_kind(restype) == _c_kind(ret), (name, ret, restype)
+        assert [_ctypes_kind(t) for t in argtypes] == [_c_kind(p) for p in params], (name, params, argtypes)
+
+
+# ctypes mirror of every struct the Python side passes through the C-ABI
+_MIRRORS = {"swb_params": engine.Params, "swb_result": engine.Result, "swb_solve_args": engine.SolveArgs,
+            "swb_round_args": engine.RoundArgs, "swb_market_args": engine.MarketArgs,
+            "swb_gavel_round_args": engine.GavelRoundArgs, "swb_sim_trace": engine.SimTrace,
+            "swb_sim_dynamic": engine.SimDynamic, "swb_sim_scn": engine.SimScn}
+
+
+def test_struct_layouts_match_header(tmp_path):
     assert engine.load_library().swb_version() >= 101
+    cc = shutil.which("cc") or shutil.which("gcc")
+    if cc is None:
+        pytest.skip("no C compiler to read the header's struct layouts")
+    lines = ["#include <stddef.h>", "#include <stdio.h>", '#include "swb200.h"', "int main(void) {"]
+    for cname, mirror in _MIRRORS.items():
+        lines.append(f'  printf("{cname} size %zu\\n", sizeof({cname}));')
+        for field, _ in mirror._fields_:
+            lines.append(f'  printf("{cname} {field} %zu\\n", offsetof({cname}, {field}));')
+    lines += ["  return 0;", "}"]
+    src, exe = tmp_path / "layouts.c", tmp_path / "layouts"
+    src.write_text("\n".join(lines) + "\n")
+    subprocess.check_call([cc, "-I", os.path.join(ROOT, "include"), str(src), "-o", str(exe)])
+    got = {}
+    for line in subprocess.check_output([str(exe)], text=True).splitlines():
+        cname, key, value = line.split()
+        got[(cname, key)] = int(value)
+    for cname, mirror in _MIRRORS.items():
+        assert C.sizeof(mirror) == got[(cname, "size")], cname
+        for field, _ in mirror._fields_:
+            assert getattr(mirror, field).offset == got[(cname, field)], (cname, field)
 
 
 def test_no_gpu_fails_loudly():
