@@ -83,7 +83,8 @@ int swb_sync(swb_ctx *ctx);
 #define SWB_OPT_RELAXED_OPTIMUM 1
 /* SWB_OPT_SOLVE_CLUSTER: CTAs per scenario on the latency path of the market solve (8 = a thread-block cluster of 8
  * CTAs shares one scenario over distributed shared memory when few scenarios of >= 512 jobs are solved; 1 = always one
- * CTA per scenario).  Process-wide.  Default 8. */
+ * CTA per scenario).  The same setting lets the fallback re-rank search of the placement start from 8 seeds over a
+ * cluster.  Per context.  Default 8. */
 #define SWB_OPT_SOLVE_CLUSTER 2
 /* Monte-Carlo (GBM) forecast inside swb_round_solve.  SWB_OPT_GBM_PATHS = P > 0: between the deterministic forecast
  * and the solve the remaining runtime of every job whose volatility model (swb_job_set_gbm) has drift or volatility

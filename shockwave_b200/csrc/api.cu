@@ -18,6 +18,7 @@ struct swb_ctx {
   DBuf wf_z, wf_x2;
   DBuf sa, su0, sR, sws, scap, sg, snF, snmax, sn, gmask, sncap, seated, scth, sths, sn0, snfc, sRr;
   int want_relaxed = 0;
+  int solve_cluster = 8;  // SWB_OPT_SOLVE_CLUSTER
   int aux_async = 0;      // SWB_OPT_ASYNC_AUX: device-output forecast / ensemble calls return without synchronising
   // ---- resident job table (by slot)
   int nslots = 0;
@@ -159,6 +160,7 @@ static int run_solve(swb_ctx *c, int S, int J, int per_scn, const swb_params *h_
   L.res = c->res.as<swb_result>();
   L.ncap = c->sncap.as<uint8_t>();
   L.sc_nfc = c->snfc.as<double>(); L.want_relaxed = c->want_relaxed;
+  L.cluster = c->solve_cluster;
   CK(cudaMemsetAsync(c->sncap.p, 0xff, n, c->st));
   swb::PlaceLaunch P;
   P.S = S; P.J = J; P.per_scn = per_scn; P.prm = L.prm; P.bfkey = bfkey; P.bfkey_fb = bfkey_fb;
@@ -166,20 +168,9 @@ static int run_solve(swb_ctx *c, int S, int J, int per_scn, const swb_params *h_
   P.sc_g = L.sc_g; P.sc_n = L.sc_n; P.sc_nmax = L.sc_nmax; P.weights = L.weights; P.E = E; P.c = cc; P.dbar = dbar;
   P.x = x; P.backfill = bf; P.nrounds = nr ? nr : c->seated.as<int32_t>(); P.ncal = ncal; P.res = L.res;
   P.xmask = xmask; P.bfmask = bfmask; P.ncap = c->sncap.as<uint8_t>();
-  // re-rank local search: O(J T^2) per cancelled cycle — on where that stays in the tens of microseconds
-  // (jobs x rounds^2 <= 256 Ki: 640 jobs at 20 rounds, 250 at 32, 64 at 64 — the reference's deployments; beyond that
-  // the priority sweep alone places the fallback schedule)
-  P.rr_items = nullptr; P.rr_iters = 0; P.rr_restarts = 0; P.prm_T = h_prm[0].future_rounds;
-  {
-    const size_t T_ = (size_t)h_prm[0].future_rounds;
-    const int cl = (S * 8 <= 144 && J <= SWB_SMEM_JOBS) ? 8 : 1;     // multi-start over a cluster (place.cu)
-    const size_t bytes = (size_t)S * cl * swb::rr_scratch_bytes(J, (int)T_);
-    P.rr_cluster = 1;
-    if (c->rr_iters > 0 && (size_t)J * T_ * T_ <= (256u << 10) && bytes <= (512u << 20)) {
-      CK(c->rr_items.need(bytes, c->st));
-      P.rr_items = c->rr_items.p; P.rr_iters = c->rr_iters; P.rr_restarts = c->rr_restarts; P.rr_cluster = cl;
-    }
-  }
+  P.plan = swb::plan_place(S, J, h_prm[0].future_rounds, c->rr_iters, c->solve_cluster);
+  if (P.plan.rerank) CK(c->rr_items.need(P.plan.rr_bytes, c->st));
+  P.rr_items = c->rr_items.p; P.rr_iters = c->rr_iters; P.rr_restarts = c->rr_restarts;
   CK(c->h_res.need(sizeof(swb_result) * S));
   const swb_result *hres = c->h_res.as<swb_result>();
   for (int pass = 0; pass < SWB_MAX_REPLAN + 1; ++pass) {
@@ -999,7 +990,7 @@ int swb_market_pgd(swb_ctx *c, const swb_market_args *a) {
 int swb_set_option(swb_ctx *c, int32_t option, int32_t value) {
   if (!c) return fail(SWB_ERR_ARG, "null ctx");
   if (option == SWB_OPT_RELAXED_OPTIMUM) { c->want_relaxed = value ? 1 : 0; return 0; }
-  if (option == SWB_OPT_SOLVE_CLUSTER) { swb::set_solve_cluster(value); swb::set_place_cluster(value); return 0; }
+  if (option == SWB_OPT_SOLVE_CLUSTER) { c->solve_cluster = (value == 8) ? 8 : 1; return 0; }
   if (option == SWB_OPT_ASYNC_AUX) { c->aux_async = value ? 1 : 0; return 0; }
   if (option == SWB_OPT_RERANK_ITERS) { c->rr_iters = value < 0 ? 0 : value; return 0; }
   if (option == SWB_OPT_RERANK_RESTARTS) { c->rr_restarts = value < 0 ? 0 : (value > 16 ? 16 : value); return 0; }

@@ -21,28 +21,6 @@
 
 namespace swb {
 
-// exclusive block scan of one int per thread (wsum: 33 ints); returns prefix, total in *tot
-__device__ __forceinline__ int gv_scan(int v, int *wsum, int *tot) {
-  int incl = v;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    int t = __shfl_up_sync(SWB_FULL, incl, o);
-    if ((threadIdx.x & 31) >= o) incl += t;
-  }
-  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
-  __syncthreads();
-  if (lane == 31) wsum[w] = incl;
-  __syncthreads();
-  int ws = lane < nw ? wsum[lane] : 0, wincl = ws;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    int t = __shfl_up_sync(SWB_FULL, wincl, o);
-    if (lane >= o) wincl += t;
-  }
-  *tot = __shfl_sync(SWB_FULL, wincl, 31);
-  return __shfl_sync(SWB_FULL, wincl - ws, w) + incl - v;
-}
-
 // a before b in the reference's queue: (priority, deficit, allocation) descending, ties in dict order
 __device__ __forceinline__ bool gv_before(const GavelLaunch &L, int w, int a, int b) {
   if (a >= L.J || b >= L.J) return a < b;          // padding sorts last
@@ -138,7 +116,7 @@ __global__ void __launch_bounds__(1024, 1) gavel_round_kernel(GavelLaunch L) {
       int lsum = 0;
       for (int q = 0; q < chs; ++q) { const int pos = p0 + q; if (pos < npad && state[pos] == 0) lsum += L.sf[ord[pos]]; }
       int tot = 0;
-      int run = gv_scan(lsum, wsum, &tot);
+      int run = block_excl_scan(lsum, wsum, &tot);
       const int left = s_left;
       int stop = 0;
       for (int q = 0; q < chs; ++q) {
@@ -167,7 +145,7 @@ __global__ void __launch_bounds__(1024, 1) gavel_round_kernel(GavelLaunch L) {
           }
         }
         int tot = 0;
-        int run = gv_scan(lsum, wsum, &tot);
+        int run = block_excl_scan(lsum, wsum, &tot);
         if (tot == 0) break;
         // the longest prefix that fits is taken at once; the first candidate beyond it does not fit what is then left
         // and is rejected by the width test of the next pass
@@ -192,7 +170,7 @@ __global__ void __launch_bounds__(1024, 1) gavel_round_kernel(GavelLaunch L) {
       int cnt = 0;
       for (int q = 0; q < chs; ++q) { const int pos = p0 + q; if (pos < npad && state[pos] == 1) ++cnt; }
       int tot = 0;
-      int off = gv_scan(cnt, wsum, &tot);
+      int off = block_excl_scan(cnt, wsum, &tot);
       for (int q = 0; q < chs; ++q) {
         const int pos = p0 + q;
         if (pos < npad && state[pos] == 1) { const int j = ord[pos]; L.sel_jobs[(size_t)ti * J + off++] = j; sched[j] |= 1; }
@@ -236,7 +214,7 @@ __global__ void __launch_bounds__(1024, 1) gavel_round_kernel(GavelLaunch L) {
       }
       __syncthreads();
       int totA = 0;
-      int offA = gv_scan(cntA, wsum, &totA);
+      int offA = block_excl_scan(cntA, wsum, &totA);
       const int baseA = s_nasg;
       for (int q = 0; q < chn; ++q) {
         const int i = n0 + q;
@@ -258,14 +236,14 @@ __global__ void __launch_bounds__(1024, 1) gavel_round_kernel(GavelLaunch L) {
         if (i < nsel && state[i] == 0 && L.sf[sel[i]] == cur && (sched[sel[i]] & 2)) { ++cntB; needB += cur; }
       }
       int totB = 0, totNeed = 0;
-      int offB = gv_scan(cntB, wsum, &totB);
-      int offNeed = gv_scan(needB, wsum, &totNeed);
+      int offB = block_excl_scan(cntB, wsum, &totB);
+      int offNeed = block_excl_scan(needB, wsum, &totNeed);
       // free workers in order: rank of every free worker
       const int chw = (nw + nt - 1) / nt, w0 = tid * chw;
       int cntF = 0;
       for (int q = 0; q < chw; ++q) { const int i = w0 + q; if (i < nw && !wbusy[i]) ++cntF; }
       int totF = 0;
-      int offF = gv_scan(cntF, wsum, &totF);
+      int offF = block_excl_scan(cntF, wsum, &totF);
       if (totNeed > totF) { if (tid == 0) s_err = 1; __syncthreads(); break; }
       const int baseB = baseA + totA;
       // every free worker with rank < totNeed goes to the job whose [offNeed, offNeed + cur) range covers the rank:

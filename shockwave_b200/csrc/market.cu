@@ -305,12 +305,7 @@ __global__ void __launch_bounds__(1024) market_dual_kernel(MarketLaunch L) {
   const int J = L.J, W = L.W, T = L.T, WT = W * T;
   const swb_params &prm = L.prm[s];
   BlockRed br(red);
-  if (threadIdx.x == 0) {
-    P.B = prm.nbases;
-    for (int b = 0; b < prm.nbases; ++b) { P.base[b] = prm.bases[b]; P.logv[b] = prm.logv[b]; }
-    for (int b = 0; b + 1 < prm.nbases; ++b)
-      P.slope[b] = (prm.logv[b + 1] - prm.logv[b]) / (prm.bases[b + 1] - prm.bases[b]);
-  }
+  if (threadIdx.x == 0) make_pwl(P, prm);
   __syncthreads();
   const double Tf = (double)L.Tfull, rs = (double)L.rscale;
   const double invJT = 1.0 / ((double)J * Tf);

@@ -18,11 +18,6 @@
 
 namespace swb {
 
-__device__ __forceinline__ unsigned long long pol_order_key(double v) {
-  unsigned long long b = (unsigned long long)__double_as_longlong(v);
-  return (b & 0x8000000000000000ull) ? ~b : (b | 0x8000000000000000ull);
-}
-
 // ---- which optimal x: the interior-point selection -------------------------------------------------------
 // These LPs are degenerate in x.  The reference solves them with interior-point codes (ECOS; Gurobi barrier for the
 // finish-time-fairness cone program, utils.py:603-685) whose iterates converge to the ANALYTIC CENTRE of the optimal
@@ -196,7 +191,7 @@ __global__ void __launch_bounds__(1024, 1) policy_kernel(PolicyLaunch L) {
     unsigned long long *key = reinterpret_cast<unsigned long long *>(smem_raw + 2 * 64 * sizeof(double));
     unsigned short *idx = reinterpret_cast<unsigned short *>(key + npad);
     for (int i = threadIdx.x; i < npad; i += blockDim.x) {
-      key[i] = i < J ? pol_order_key(L.coef[i] / L.sf[i]) : 0ull;
+      key[i] = i < J ? order_key(L.coef[i] / L.sf[i]) : 0ull;
       idx[i] = (unsigned short)(i < J ? i : 0xffff);
     }
     __syncthreads();

@@ -28,7 +28,10 @@
 namespace swb {
 
 
-// scratch of one search (global memory, L2 resident): sized by rr_scratch_bytes()
+#define RR_MAXCLS 4
+#define RR_ITEMJOBS 8
+
+// scratch of one search (global memory, L2 resident), carved by rr_carve()
 struct RrScratch {
   double *wj;              // [J] w_j = prio_j / n_j (0: job not movable)
   double *cost;            // [RR_MAXCLS][N*N] dense edge costs, N = T + 1, row u -> column v
@@ -41,33 +44,37 @@ struct RrScratch {
   int *bki;                // [T] its idle GPUs
   double *wn;              // [J] w_j x noise of the current phase (what the edge costs are built from)
   unsigned short *ord;     // [J] movable jobs grouped by width class, ascending job index inside a class
+  size_t hot_bytes;        // w_j and the dense cost matrices: the head of the scratch, or of a copy in shared memory
 };
 #define RR_MAXBAN 64
 #define RR_REV 0x8000u     // job entry of an item: this job moves AGAINST the edge (v -> u)
-// hot: w_j and the dense cost matrices in SHARED memory (hot != null), else in the global scratch
-__device__ __forceinline__ RrScratch rr_carve(unsigned char *base, unsigned char *hot, int J, int T) {
+// Carves the scratch of one search at `base` (256-byte aligned) and returns its size, a multiple of 256 bytes.  With
+// hot != null (16-byte aligned, hot_bytes long) w_j and the dense cost matrices are read from there instead.
+// Called with base = hot = nullptr it only sizes.
+__host__ __device__ __forceinline__ size_t rr_carve(RrScratch &s, unsigned char *base, unsigned char *hot, int J,
+                                                    int T) {
   const size_t N = (size_t)T + 1, TT = (size_t)T * T;
-  RrScratch s;
-  s.wj = reinterpret_cast<double *>(base); base += (size_t)J * 8;
-  s.cost = reinterpret_cast<double *>(base); base += RR_MAXCLS * N * N * 8;
-  s.jobs = reinterpret_cast<unsigned short *>(base); base += RR_MAXCLS * TT * RR_ITEMJOBS * 2;
-  s.nj = base; base += RR_MAXCLS * TT;
-  base = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(base) + 15) & ~uintptr_t(15));
-  s.log = reinterpret_cast<int *>(base); base += N * RR_ITEMJOBS * 8;
-  s.swc = reinterpret_cast<double *>(base); base += N * N * 8;
-  s.swj = reinterpret_cast<unsigned short *>(base); base += N * N * 8;
-  base = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(base) + 15) & ~uintptr_t(15));
-  s.bkx = reinterpret_cast<unsigned long long *>(base); base += (size_t)J * 16;
-  s.bki = reinterpret_cast<int *>(base); base += N * 4;
-  base = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(base) + 15) & ~uintptr_t(15));
-  s.wn = reinterpret_cast<double *>(base); base += (size_t)J * 8;
-  s.ord = reinterpret_cast<unsigned short *>(base);
+  unsigned char *p = base;
+  s.wj = reinterpret_cast<double *>(p); p += (size_t)J * 8;
+  s.cost = reinterpret_cast<double *>(p); p += RR_MAXCLS * N * N * 8;
+  s.hot_bytes = (size_t)(p - base);
+  s.jobs = reinterpret_cast<unsigned short *>(p); p += RR_MAXCLS * TT * RR_ITEMJOBS * 2;
+  s.nj = p; p += RR_MAXCLS * TT;
+  p = align16(p);
+  s.log = reinterpret_cast<int *>(p); p += N * RR_ITEMJOBS * 8;
+  s.swc = reinterpret_cast<double *>(p); p += N * N * 8;
+  s.swj = reinterpret_cast<unsigned short *>(p); p += N * N * 8;
+  p = align16(p);
+  s.bkx = reinterpret_cast<unsigned long long *>(p); p += (size_t)J * 16;
+  s.bki = reinterpret_cast<int *>(p); p += N * 4;
+  p = align16(p);
+  s.wn = reinterpret_cast<double *>(p); p += (size_t)J * 8;
+  s.ord = reinterpret_cast<unsigned short *>(p); p += (size_t)J * 2;
   if (hot) {
-    hot = reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(hot) + 15) & ~uintptr_t(15));
     s.wj = reinterpret_cast<double *>(hot);
     s.cost = s.wj + J;
   }
-  return s;
+  return ((size_t)(p - base) + 255) & ~(size_t)255;
 }
 
 __device__ __forceinline__ double rr_noise(int j, unsigned seed) {
@@ -261,7 +268,8 @@ __device__ __noinline__ int rr_local_search(unsigned char *scratch, unsigned cha
   __shared__ int s_cls[RR_MAXCLS], s_ncls, s_found, s_len[RR_MAXCLS], s_ban[RR_MAXBAN], s_nban, s_off[RR_MAXCLS + 1];
   __shared__ double s_part[32];
   __shared__ int s_parti[32];
-  const RrScratch S = rr_carve(scratch, hot, J, T);
+  RrScratch S;
+  rr_carve(S, scratch, hot, J, T);
   const int N = T + 1;
   for (int j = threadIdx.x; j < J; j += blockDim.x)
     S.wj[j] = (nplan[j] > 0 && remn[j] == 0 && isfinite(prio[j])) ? prio[j] / (double)nplan[j] : 0.0;

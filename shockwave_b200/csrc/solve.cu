@@ -174,10 +174,9 @@ __device__ __forceinline__ double rem_of(const Ctx &c, int j, int n) {
   return fmax(0.0, c.Rsec[j] - done);
 }
 
-// weighted PWL-log utility of n rounds.  A job that completes inside the window gets plog(1) = 0
-// EXACTLY: the fallback priorities reach 1e20 and would amplify a 1-ulp error in u to O(1).
+// weighted PWL-log utility of n rounds
 __device__ __forceinline__ double util_of(const Ctx &c, int j, int n) {
-  const double u = (c.D * (double)n >= c.cap[j]) ? 1.0 : fma(c.a[j], (double)n, c.u0[j]);
+  const double u = util_u(c.a[j], c.u0[j], c.cap[j], c.D, n);
   return c.ws[j] * plog(*c.P, u);
 }
 
@@ -443,12 +442,7 @@ __global__ void __launch_bounds__(NT, 1) solve_kernel(SolveLaunch L) {
   for (int b = 0; b < 8; ++b)
     c.sl[b] = (b + 1 < B) ? (float)((prm.logv[b + 1] - prm.logv[b]) / (prm.bases[b + 1] - prm.bases[b])) : -INFINITY;
 
-  if (threadIdx.x == 0) {
-    P->B = B;
-    for (int b = 0; b < B; ++b) { P->base[b] = prm.bases[b]; P->logv[b] = prm.logv[b]; }
-    for (int b = 0; b + 1 < B; ++b)
-      P->slope[b] = (prm.logv[b + 1] - prm.logv[b]) / (prm.bases[b + 1] - prm.bases[b]);
-  }
+  if (threadIdx.x == 0) make_pwl(*P, prm);
   __syncthreads();
 
   const size_t jo = L.per_scn ? so : 0;
@@ -531,8 +525,7 @@ __global__ void __launch_bounds__(NT, 1) solve_kernel(SolveLaunch L) {
       }
       float th = -1.0f;
       if (n0 < nmax) {
-        const double u1 = (D * (double)(n0 + 1) >= cap) ? 1.0 : fma(a, (double)(n0 + 1), u0);
-        const double u_0 = (D * (double)n0 >= cap) ? 1.0 : fma(a, (double)n0, u0);
+        const double u1 = util_u(a, u0, cap, D, n0 + 1), u_0 = util_u(a, u0, cap, D, n0);
         th = (float)((plog(*P, u1) - plog(*P, u_0)) / a);
       }
       c.t.n0[j * B + bs] = (uint8_t)n0;
@@ -710,10 +703,6 @@ __global__ void __launch_bounds__(NT, 1) solve_kernel(SolveLaunch L) {
   if constexpr (CL > 1) cg::this_cluster().sync();   // nobody leaves while its exchange slots may still be read
 }
 
-static int g_solve_cl = 8;      // CTAs per scenario on the latency path (SWB_OPT_SOLVE_CLUSTER = 1 switches the cluster off)
-
-void set_solve_cluster(int v) { g_solve_cl = (v == 8) ? 8 : 1; }
-
 template <class K>
 static cudaError_t set_smem_attr(K kern, int static_bytes) {
   return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SWB_MAX_DYN_SMEM - static_bytes);
@@ -736,7 +725,7 @@ cudaError_t launch_solve(const SolveLaunch &L, cudaStream_t st, int nbases) {
   }
   // Latency path: few scenarios of many jobs leave most of the 148 SMs idle with one CTA per scenario — a cluster of
   // 8 CTAs (portable size, same die) shares one scenario over distributed shared memory instead.
-  if (L.jobs_in_smem && g_solve_cl == 8 && L.J >= 512 && L.S * 8 <= 144) {
+  if (L.jobs_in_smem && L.cluster == 8 && L.J >= 512 && L.S * 8 <= 144) {
     const int Jc = ((((L.J + 7) / 8) + 31) & ~31);
     const size_t smem = smem_fixed + (size_t)Jc * (2 * sizeof(double) + 5 * (size_t)nbases + 3);
     int nt = Jc < 512 ? Jc : 512;

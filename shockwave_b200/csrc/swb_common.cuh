@@ -12,6 +12,11 @@
 
 namespace swb {
 
+// the first 16-byte boundary at or after p (shared-memory and scratch carve-ups)
+__host__ __device__ __forceinline__ unsigned char *align16(unsigned char *p) {
+  return reinterpret_cast<unsigned char *>((reinterpret_cast<uintptr_t>(p) + 15) & ~uintptr_t(15));
+}
+
 // Piecewise-linear log through (base_b, logv_b): the reference's SOS2 model (shockwave.py:384-419)
 // evaluated directly — for a concave maximise the LP picks adjacent breakpoints, so
 // plog(u) == min_b(slope_b * (u - base_b) + logv_b) on [0,1].
@@ -30,6 +35,27 @@ __device__ __forceinline__ double plog(const Pwl &P, double u) {
   int b = 0;
   for (int i = 1; i < P.B - 1; ++i) b = (u >= P.base[i]) ? i : b;
   return fma(P.slope[b], u - P.base[b], P.logv[b]);
+}
+
+// the breakpoints of a scenario and the slopes between them
+__device__ __forceinline__ void make_pwl(Pwl &P, const swb_params &prm) {
+  const int B = prm.nbases;
+  P.B = B;
+  for (int b = 0; b < B; ++b) { P.base[b] = prm.bases[b]; P.logv[b] = prm.logv[b]; }
+  for (int b = 0; b + 1 < B; ++b)
+    P.slope[b] = (prm.logv[b + 1] - prm.logv[b]) / (prm.bases[b + 1] - prm.bases[b]);
+}
+
+// utility u of a job after n rounds: u0 + a n, or exactly 1 once the job completes inside the window (the fallback
+// priorities reach 1e20 and would amplify a 1-ulp error in u to O(1))
+__device__ __forceinline__ double util_u(double a, double u0, double cap, double D, int n) {
+  return (D * (double)n >= cap) ? 1.0 : fma(a, (double)n, u0);
+}
+
+// unsigned key that sorts like the double it is made from (ascending)
+__device__ __forceinline__ unsigned long long order_key(double v) {
+  unsigned long long b = (unsigned long long)__double_as_longlong(v);
+  return (b & 0x8000000000000000ull) ? ~b : (b | 0x8000000000000000ull);
 }
 
 __device__ __forceinline__ int warp_sum(int v) {
@@ -56,6 +82,32 @@ __device__ __forceinline__ double warp_min(double v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v = fmin(v, __shfl_xor_sync(SWB_FULL, v, o));
   return v;
+}
+
+// exclusive block scan of one int per thread; returns the exclusive prefix, total in *tot.
+// wsum needs 33 ints.  Two barriers; the 32 warp totals are scanned by warp 0 with shuffles.
+__device__ __forceinline__ int block_excl_scan(int v, int *wsum, int *tot) {
+  int incl = v;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    int t = __shfl_up_sync(SWB_FULL, incl, o);
+    if ((threadIdx.x & 31) >= o) incl += t;
+  }
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
+  __syncthreads();  // protect wsum from the previous use
+  if (lane == 31) wsum[w] = incl;
+  __syncthreads();
+  // every warp scans the (<= 32) warp totals redundantly: no third barrier
+  int ws = lane < nw ? wsum[lane] : 0;
+  int wincl = ws;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    int t = __shfl_up_sync(SWB_FULL, wincl, o);
+    if (lane >= o) wincl += t;
+  }
+  *tot = __shfl_sync(SWB_FULL, wincl, 31);
+  const int off = __shfl_sync(SWB_FULL, wincl - ws, w);
+  return off + incl - v;
 }
 
 // Block reductions with ONE __syncthreads each: two scratch rows used alternately (ping-pong), so

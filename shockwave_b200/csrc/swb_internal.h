@@ -112,7 +112,20 @@ struct SolveLaunch {
   const uint8_t *ncap; // [S][J] per-job cap on the round count from packing feedback (255 = none)
   double *weights;   // [S][J] out, may be null
   swb_result *res;   // device [S]
+  int cluster;       // SWB_OPT_SOLVE_CLUSTER: 8 lets few scenarios of many jobs share each over a cluster of 8 CTAs
 };
+
+// How one call's placement is launched, decided once by plan_place (place.cu).
+struct PlacePlan {
+  int rerank;             // 1: the fallback re-rank search runs
+  int cluster;            // CTAs per scenario: 8 (the search starts from 8 seeds over a thread-block cluster) or 1
+  int hot_smem;           // 1: the search's hot arrays (w_j, dense edge costs) sit in shared memory, 0: in its scratch
+  int threads;            // per CTA
+  size_t smem;            // dynamic shared memory per CTA
+  size_t rr_region;       // scratch of one search
+  size_t rr_bytes;        // scratch of the launch: S x cluster regions (0: search off)
+};
+PlacePlan plan_place(int S, int J, int T, int rr_iters, int cluster_opt);
 
 struct PlaceLaunch {
   int S, J, per_scn;
@@ -130,31 +143,14 @@ struct PlaceLaunch {
   int32_t *ncal;          // [S][J] out, may be null: rounds with idle GPUs in which the job is unscheduled
   swb_result *res;        // device [S] (status in, objective/shortfall updated)
   uint8_t *ncap;          // [S][J] in/out, may be null: per-job count caps for the next pass (packing feedback)
-  void *rr_items;         // scratch of the re-rank local search, S x rr_cluster x rr_scratch_bytes(J, T) (null: off)
+  void *rr_items;         // scratch of the re-rank local search, plan.rr_bytes
   int rr_iters;           // cycle-cancelling budget per scenario
   int rr_restarts;        // perturb-and-continue rounds after the first local optimum (iterated local search)
-  int prm_T;              // future_rounds of the call (host copy, for sizing)
-  int rr_cluster;         // 8: rr_items holds 8 regions per scenario (multi-start over a thread-block cluster), else 1
-  int rr_hot_smem;        // 1: the search's hot arrays (w_j, dense edge costs) sit in shared memory, 0: in rr_items
+  PlacePlan plan;
 };
 
 cudaError_t launch_solve(const SolveLaunch &L, cudaStream_t st, int nbases);
-void set_solve_cluster(int ctas_per_scenario);
-// scratch of one re-rank local search (rerank.cuh): w_j, dense edge costs per width class, best items per (class, pair)
-#define RR_MAXCLS 4
-#define RR_ITEMJOBS 8
-__host__ __device__ inline size_t rr_scratch_bytes(int J, int T) {
-  const size_t N = (size_t)T + 1, TT = (size_t)T * T;
-  size_t b = (size_t)J * 8 + RR_MAXCLS * N * N * 8 + RR_MAXCLS * TT * RR_ITEMJOBS * 2 + RR_MAXCLS * TT;
-  b = (b + 15) & ~(size_t)15;
-  b += N * RR_ITEMJOBS * 8;          // move log of the cycle being applied (job, from, to)
-  b += N * N * 16;                   // best swap-into-idle move of every ordered pair of rounds (cost, jobs, class)
-  b += (size_t)J * 16 + N * 4 + 16;  // best schedule so far of the iterated search (round masks, idle GPUs)
-  b += (size_t)J * 8 + (size_t)J * 2 + 32;   // noised weights of the current phase, job order by width class
-  return (b + 255) & ~(size_t)255;
-}
 cudaError_t launch_place(const PlaceLaunch &L, cudaStream_t st, unsigned long long *gmask);
-void set_place_cluster(int ctas_per_scenario);
 
 struct ForecastLaunch {
   int J;

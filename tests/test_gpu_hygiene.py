@@ -105,3 +105,34 @@ def test_cluster_solve_equals_single_cta_solve(engine, J, G, T, k):
         assert np.array_equal(a["x"], b["x"])
         assert abs(a["results"][0]["objective"] - b["results"][0]["objective"]) <= 1e-9 * abs(a["results"][0]["objective"])
     engine.set_option(6, 400)
+
+
+def test_solve_cluster_option_belongs_to_its_engine(engine):
+    """SWB_OPT_SOLVE_CLUSTER = 1 on one Engine leaves another Engine's fallback placement on its 8-start re-rank search
+    (thread-block cluster): a recorded canonical fallback solve whose best start is not start 0 (flags >> 20) gives the
+    same schedule and flags before and after the option is set elsewhere."""
+    from shockwave_b200 import Engine
+    T, G, D = fx.TACC["T"], fx.TACC["G"], fx.TACC["D"]
+
+    def run(s):
+        prm = make_params(G, T, D, fx.TACC["k"], fx.TACC["lam"], fx.TACC["rhomax"], fx.BASES, fx.ORIGIN,
+                          round_ptr=s["round_ptr"])
+        return engine.solve(prm, s["g"], s["E"], s["c"], s["dbar"], s["rem"], s["ftobj"], bfkey=s["rem"])
+
+    cases = []
+    for i in range(fx.n_solves()):
+        s = fx.solve(i)
+        if s["status"] == om.STATUS_FALLBACK:
+            out = run(s)
+            if out["results"][0]["flags"] >> 20:
+                cases.append((s, out))
+    assert cases, "no recorded fallback solve is won by a noised start"
+    other = Engine(0)
+    try:
+        other.set_option(2, 1)
+        for s, before in cases[:8]:
+            after = run(s)
+            assert after["results"][0]["flags"] == before["results"][0]["flags"]
+            assert np.array_equal(after["x"], before["x"])
+    finally:
+        other.close()
